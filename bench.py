@@ -2,7 +2,7 @@
 """Headline benchmark: GTEPS of one GAT layer on a Reddit-shape synthetic graph, executed from
 the ISA program the reference's compiler.py -> interpreter.py emit (tests/golden/isa), on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU); the graph is partitioned by destination range
 (balanced by edges), each layer all-gathers Z and er over NCCL.  Prints ONE JSON line (rank 0).
@@ -11,6 +11,10 @@ A step = one full GAT layer (ops 0-13 of genGraphOP.py:49-62): GEMM X.W with the
 projections, single-pass edge softmax + aggregation + ELU.  ``value`` = E / step time with the
 inputs resident in HBM; ``e2e`` = the same through ``execute()`` with HOST (pinned) features
 copied in and the result copied out inside the timed region.
+
+``--dump-outputs DIR`` writes the last timed step's layer output (``output.npy``) and the global row ids it
+holds (``output_rows.npy``): every row, or a fixed seeded sample of rows beyond 64 MB.  With N > 1 only rank
+0's destination rows are written; which rows rank 0 owns depends on N, so compare dumps taken with the same N.
 """
 from __future__ import annotations
 
@@ -327,6 +331,22 @@ def parity_big(P, torch, y_h, ip_s, ix_s, rows_sel, edge_w_rows, x_d, w_d, z_loc
     return rep
 
 
+DUMP_BYTES = 64 * 10**6 - 4096      # --dump-outputs budget, .npy headers included
+
+
+def dump_outputs(out_dir, y, row0):
+    """--dump-outputs: ``y`` (rank 0's output rows, global ids from ``row0``; every row when N = 1) as float32, every
+    row when it fits DUMP_BYTES, else the same seeded sample of rows on every run of the same shape."""
+    rows, cols = int(y.shape[0]), int(y.shape[1])
+    keep = min(rows, DUMP_BYTES // (cols * 4 + 8))
+    pick = np.arange(rows) if keep == rows else np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+    import torch
+    vals = y[torch.from_numpy(pick).to(y.device)].float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "output.npy"), vals)
+    np.save(os.path.join(out_dir, "output_rows.npy"), (pick + row0).astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------
@@ -358,7 +378,13 @@ def main():
     ap.add_argument("--dtype", default="f32", choices=["f32", "bf16"],
                     help="bf16 = bf16 STORAGE MODE: the gathered table Z in bf16, fp32 accumulation (its own tolerance: "
                          "rtol 2e-2, atol 1e-2 rowscale); never the headline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the layer output of the last timed step to DIR/output.npy (float32; rank 0's rows) and "
+                         "the global row ids it holds to DIR/output_rows.npy (float64): every row when both fit "
+                         "64 MB, else a fixed seeded sample of rows, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     wl = resolve_workload(args.workload)
     rank = int(os.environ.get("RANK", "0"))
@@ -366,6 +392,8 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the GPU path's output; --impl reference times a host sample")
         if rank == 0:
             run_reference_arm(args, wl)
         return
@@ -531,6 +559,8 @@ def main():
     barrier()
     elapsed_ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:      # before more steps run: a replayed graph reuses its output buffer
+        dump_outputs(args.dump_outputs, y, r0)
     t = torch.tensor([elapsed_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -244,6 +244,59 @@ def test_bench_refuses_to_run_the_gpu_arm_without_a_gpu():
     assert r.returncode != 0 and "no CPU fallback" in (r.stderr + r.stdout)
 
 
+def _bench_module():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(REPO, "bench.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
+@pytest.mark.parametrize("rows,cols", [(300, 128), (232965, 128), (1 << 16, 256)])
+def test_bench_dump_outputs_stays_in_budget_and_samples_the_same_rows(rows, cols, tmp_path):
+    """--dump-outputs: every row when they fit 64 MB, else the same seeded row sample on every call; values are the
+    rows the ids name (offset by the rank's first row)."""
+    import numpy as np
+    import torch
+    bench = _bench_module()
+    y = torch.arange(rows * cols, dtype=torch.float32).reshape(rows, cols) % 1021
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), y, 7)
+    assert sum(os.path.getsize(p) for p in tmp_path.glob("a/*")) <= 64 * 10**6
+    vals, ids = np.load(tmp_path / "a" / "output.npy"), np.load(tmp_path / "a" / "output_rows.npy")
+    assert vals.dtype == np.float32 and ids.dtype == np.float64 and vals.shape[1] == cols
+    assert np.array_equal(vals, y.numpy()[ids.astype(np.int64) - 7])
+    assert np.all(np.diff(ids) > 0) and (vals.shape[0] == rows) == (rows * (cols * 4 + 8) <= 64 * 10**6 - 4096)
+    assert np.array_equal(ids, np.load(tmp_path / "b" / "output_rows.npy"))
+    assert np.array_equal(vals, np.load(tmp_path / "b" / "output.npy"))
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_writes_the_benchmarked_layer(tmp_path):
+    """bench.py --dump-outputs on the Cora GAT layer: the whole output (2708 x 128, rows 0..N-1) equals the fp64
+    oracle's GAT layer on the bench's seeded inputs, within the fp32 error scale smoke() uses."""
+    import subprocess
+    import sys
+    import numpy as np
+    from oracle import gta_oracle as O
+    from gta_graph_tensor_acclelrator_for_general_gnn_b200 import synthetic
+    subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--workload", "cora-gat", "--steps", "2",
+                    "--warmup", "3", "--no-e2e", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                   capture_output=True, text=True, timeout=600, check=True)
+    vals, ids = np.load(tmp_path / "output.npy"), np.load(tmp_path / "output_rows.npy")
+    n, _, fin = synthetic.SHAPES["cora"]
+    assert vals.shape == (n, 128) and vals.dtype == np.float32 and np.all(np.isfinite(vals))
+    assert np.array_equal(ids, np.arange(n, dtype=np.float64))
+    g = synthetic.shape_graph("cora")
+    x, w, al, ar = synthetic.gat_tensors(n, fin, 128, 4, seed=0)
+    indptr, indices, _ = O.csr_build(g.dst, g.src, n)
+    ref = O.gat_layer(indptr, indices, x, w, al, ar)
+    zscale = np.abs(x).astype(np.float64) @ np.abs(w).astype(np.float64)
+    scale = O.segment_sum(O.head_broadcast(ref["alpha"], 128) * zscale[indices], indptr)
+    err = np.abs(vals - ref["Y"]) / (1e-5 * np.abs(ref["Y"]) + 1e-5 * scale + 1e-30)
+    assert err.max() <= 1.0, f"dumped output {err.max():.2f}x the tolerance away from the fp64 oracle"
+
+
 @pytest.mark.parametrize("n", [1, 2, 4, 8])
 def test_committed_bench_lines_carry_the_contract_keys(n):
     """profiles/r01_bench_n*.json: the GPU arm's lines as measured on the box (what DESIGN.md quotes)."""
