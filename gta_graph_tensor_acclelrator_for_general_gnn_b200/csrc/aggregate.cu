@@ -12,9 +12,11 @@
 // lanes.  Wider rows (F > 128) are covered by blockIdx.y feature windows of 128.  Source ids (and
 // scalar edge weights) are read once per group, coalesced and streaming (L1 no-allocate, L2
 // evict_first), then handed round the group by shuffle / shared memory.  Gathered rows use the
-// read-only path without L1 allocation (no reuse inside an SM); L2 residency comes from the
-// column-block order of the work list.  kUnroll independent row loads are in flight per lane and a
-// full batch runs without a single predicate.
+// coherent path without L1 allocation (no reuse inside an SM) and with an L2 evict_last policy; L2
+// residency comes from the column-block order of the work list.  Not the non-coherent (.nc) path: in
+// an exchange the copy CTAs write the peers' slots of the table during the same launch, and .nc is
+// only valid for data that no thread writes while the kernel runs.  kUnroll independent row loads are
+// in flight per lane and a full batch runs without a single predicate.
 //
 // Rows that own several items (long rows cut at `chunk` edges, and every row when the table is walked
 // in column blocks) form a CHAIN in slot order: an item reduces its own edges first, then waits for
@@ -49,9 +51,7 @@ aggregate_kernel(const WorkList wl, const Exchange ex, const float* __restrict__
   constexpr int kWindow = LANES * KP * V;          // features one pass of a group covers
   constexpr int kEdges = kAggUnroll;      // edges whose loads (V each) are in flight together
   __shared__ __align__(16) uint2 s_a[kAggWarps][32];        // per warp: {source id, weight} of the staged batch
-#if GTA_ITEM_PREFETCH
   __shared__ __align__(16) NextItem s_next[kAggWarps][32 / LANES];
-#endif
   if (ex.world > 1 && blockIdx.y == 0 && blockIdx.x < ex.copy_ctas) {
     exchange_pull(ex, blockIdx.x);          // these CTAs move the peers' slots; everybody else reduces
     return;
@@ -70,13 +70,11 @@ aggregate_kernel(const WorkList wl, const Exchange ex, const float* __restrict__
   for (int v = 0; v < V; ++v) on[v] = fo + v * LANES * KP < f;
   const char* xf = reinterpret_cast<const char*>(x + (on[0] ? fo : 0));
 
-  ItemCursor cur = cursor_begin<LANES>(wl, ex, counter, lane);
+  const ItemCursor first = cursor_begin<LANES>(wl, ex, counter, lane);
   int32_t landed = 0;          // exchange_gate: highest peer slot this lane has seen complete
   const int head = (WKIND == 2 && on[0]) ? fo / (f / wh) : 0;
   // what an item needs before its first batch (see NextItem): record, first ids (and scalar weights), the row's
   // denominator, and -- in an exchange -- its last id, which names the highest slot it touches
-  int4 it = make_int4(0, 0, 0, -1);
-  bool have = false;
   int idx_nxt = 0, last_src = 0;
   float w_nxt = 0.f, den = 1.f;
   auto request_inputs = [&](const int4& t, bool hv) {
@@ -92,36 +90,12 @@ aggregate_kernel(const WorkList wl, const Exchange ex, const float* __restrict__
     if (DIV && hv) den = rowden[int64_t(t.x) * wh + head];
     last_src = (ex.world > 1 && cnt > 0) ? __ldg(ib + cnt - 1) : 0;
   };
-#if GTA_ITEM_PREFETCH
-  NextItem* nx = &s_next[threadIdx.x >> 5][lane / LANES];
-  {
-    const int64_t group = int64_t(cur.first) + lane / LANES;
-    have = group < wl.num_items;
-    if (have) it = __ldg(wl.items + group);
-    request_inputs(it, have);
-  }
-#endif
-  while (cur.first < wl.num_items) {
-#if GTA_ITEM_PREFETCH
-    ItemCursor nxt = cur;
-    cursor_next<LANES>(nxt, wl, counter, lane);
-    const int64_t ngroup = int64_t(nxt.first) + lane / LANES;
-    const bool nhave = nxt.first < wl.num_items && ngroup < wl.num_items;
-    if (l == 0) {
-      if (nhave) cp_async_16(&nx->item, wl.items + ngroup);
-      if (have && it.w >= 0) {
-        cp_async_4(&nx->s0, wl.row_slots + it.x);
-        cp_async_4(&nx->s1, wl.row_slots + it.x + 1);
-      }
-    }
-#else
-    {
-      const int64_t group = int64_t(cur.first) + lane / LANES;
-      have = group < wl.num_items;
-      it = have ? __ldg(wl.items + group) : make_int4(0, 0, 0, -1);
-      request_inputs(it, have);
-    }
-#endif
+  ItemStage<LANES> stage(wl, first, lane, &s_next[threadIdx.x >> 5][lane / LANES]);
+  request_inputs(stage.it, stage.have);
+  while (stage.cur.first < wl.num_items) {
+    stage.claim(wl, counter, lane);
+    const int4 it = stage.it;
+    const bool have = stage.have;
     const bool active = have && on[0];
     const int count = have ? it.z : 0;
     const int max_count = (LANES == 32) ? count : warp_max_i32(count);
@@ -224,57 +198,31 @@ aggregate_kernel(const WorkList wl, const Exchange ex, const float* __restrict__
       __syncwarp();
     }
     const bool chained = have && it.w >= 0;
-#if GTA_ITEM_PREFETCH
-    cp_async_wait_all();
-    __syncwarp();
-    const int4 itn = nhave ? nx->item : make_int4(0, 0, 0, -1);
-    const int slot0 = chained ? nx->s0 : 0, slot1 = chained ? nx->s1 : 0;
-    __syncwarp();          // everybody has read the staging entry before lane 0 of the group overwrites it
-    request_inputs(itn, nhave);
-#endif
-    for_groups_in_order<LANES>(lane, chained, [&]() {
-      bool last = true;
-      if (chained) {
-#if GTA_ITEM_PREFETCH
-        const int s0 = slot0, s1 = slot1;
-#else
-        const int s0 = __ldg(wl.row_slots + it.x), s1 = __ldg(wl.row_slots + it.x + 1);
-#endif
-        last = it.w == s1 - 1;
-        if (it.w != s0) {
-          if (l == 0) chain_wait(flags + it.w - 1);
-          __syncwarp(group_mask<LANES>(lane));
+    const int4 next = stage.land(chained);
+    request_inputs(next, stage.next_have);
+    chain_step<LANES>(flags, lane, it, chained, [&]() { return stage.slots; },
+        [&](int prev) {
 #pragma unroll
           for (int v = 0; v < V; ++v) {
             if (have && on[v]) {
               float p[KP];
-              ld_state<KP>(wl.partials + int64_t(it.w - 1) * f + fo + v * LANES * KP, p);
+              ld_state<KP>(wl.partials + int64_t(prev) * f + fo + v * LANES * KP, p);
 #pragma unroll
               for (int c = 0; c < KP; ++c) acc[v][c] = p[c] + acc[v][c];
             }
           }
-        }
-        if (!last) {
+        },
+        [&](int slot) {
 #pragma unroll
           for (int v = 0; v < V; ++v)
-            if (have && on[v]) st_state<KP>(wl.partials + int64_t(it.w) * f + fo + v * LANES * KP, acc[v]);
-          __syncwarp(group_mask<LANES>(lane));          // the group's stores happen-before lane 0's release
-          if (l == 0) chain_publish(flags + it.w);
-        }
-      }
-      if (last) {
+            if (have && on[v]) st_state<KP>(wl.partials + int64_t(slot) * f + fo + v * LANES * KP, acc[v]);
+        },
+        [&]() {
 #pragma unroll
-        for (int v = 0; v < V; ++v)
-          if (have && on[v]) st_out<KP>(out + int64_t(it.x) * ldo + fo + v * LANES * KP, acc[v], 1.f, epilogue);
-      }
-    });
-#if GTA_ITEM_PREFETCH
-    cur = nxt;
-    it = itn;
-    have = nhave;
-#else
-    cursor_next<LANES>(cur, wl, counter, lane);
-#endif
+          for (int v = 0; v < V; ++v)
+            if (have && on[v]) st_out<KP>(out + int64_t(it.x) * ldo + fo + v * LANES * KP, acc[v], 1.f, epilogue);
+        });
+    stage.advance(next);
   }
 }
 
@@ -318,7 +266,7 @@ edge_sum_kernel(const WorkList wl, const Exchange ex, const float* __restrict__ 
     const int count = have ? it.z : 0;
     const int max_count = (LANES == 32) ? count : warp_max_i32(count);
     const int32_t* idx_base = wl.indices + it.y;
-    const float* xf = HAS_X ? x + (active ? fo : 0) : nullptr;
+    const char* xf = HAS_X ? reinterpret_cast<const char*>(x + (active ? fo : 0)) : nullptr;
     const float* ef = HAS_E ? edge + int64_t(it.y) * lde + (active ? fo : 0) : nullptr;
     float4 r4 = make_float4(0.f, 0.f, 0.f, 0.f);
     if (active && rowterm != nullptr) r4 = __ldg(reinterpret_cast<const float4*>(rowterm + int64_t(it.x) * ldr + fo));
@@ -342,7 +290,7 @@ edge_sum_kernel(const WorkList wl, const Exchange ex, const float* __restrict__ 
           const bool ok = active && (j + u) < n;
           xv[u] = make_float4(0.f, 0.f, 0.f, 0.f);
           ev[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (HAS_X && ok) xv[u] = ld_row_f32x4(row_ptr(xf, mine[(j + u) & (LANES - 1)], row_bytes), pol_keep);
+          if (HAS_X && ok) xv[u] = F32x4::unpack(F32x4::load(row_addr(xf, mine[(j + u) & (LANES - 1)], row_bytes), pol_keep));
           if (HAS_E && ok) ev[u] = ld_gather_f32x4(ef + int64_t(base + j + u) * lde, pol_stream);          // streamed: read once, evict first
         }
 #pragma unroll
@@ -358,27 +306,16 @@ edge_sum_kernel(const WorkList wl, const Exchange ex, const float* __restrict__ 
       if (HAS_X) __syncwarp();
     }
     const bool chained = have && it.w >= 0;
-    for_groups_in_order<LANES>(lane, chained, [&]() {
-      bool last = true;
-      if (chained) {
-        const int s0 = __ldg(wl.row_slots + it.x), s1 = __ldg(wl.row_slots + it.x + 1);
-        last = it.w == s1 - 1;
-        if (it.w != s0) {
-          if (l == 0) chain_wait(flags + it.w - 1);
-          __syncwarp(group_mask<LANES>(lane));
+    chain_step<LANES>(flags, lane, it, chained,
+        [&]() { return make_int2(__ldg(wl.row_slots + it.x), __ldg(wl.row_slots + it.x + 1)); },
+        [&](int prev) {
           if (active) {
-            const float4 p = ld_state_f32x4(wl.partials + int64_t(it.w - 1) * f + fo);
+            const float4 p = ld_state_f32x4(wl.partials + int64_t(prev) * f + fo);
             acc.x = p.x + acc.x; acc.y = p.y + acc.y; acc.z = p.z + acc.z; acc.w = p.w + acc.w;
           }
-        }
-        if (!last) {
-          if (active) *reinterpret_cast<float4*>(wl.partials + int64_t(it.w) * f + fo) = acc;
-          __syncwarp(group_mask<LANES>(lane));          // the group's stores happen-before lane 0's release
-          if (l == 0) chain_publish(flags + it.w);
-        }
-      }
-      if (last && active) st_stream_f32x4(out + int64_t(it.x) * ldo + fo, epilogue4(acc, 1.f, epilogue));
-    });
+        },
+        [&](int slot) { if (active) *reinterpret_cast<float4*>(wl.partials + int64_t(slot) * f + fo) = acc; },
+        [&]() { if (active) st_stream_f32x4(out + int64_t(it.x) * ldo + fo, epilogue4(acc, 1.f, epilogue)); });
     cursor_next<LANES>(cur, wl, counter, lane);
   }
 }
@@ -396,7 +333,7 @@ gather_peak_kernel(const float* __restrict__ table, uint32_t rows, uint32_t row_
   const int lane = threadIdx.x & 31;
   const int l = lane % lanes_per_row;
   const uint64_t group = (uint64_t(blockIdx.x) * blockDim.x + threadIdx.x) / lanes_per_row;
-  const float* base = table + 4 * l;
+  const char* base = reinterpret_cast<const char*>(table + 4 * l);
   float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
   uint32_t state = uint32_t(group * 2654435761u) | 1u;
   for (int64_t i = 0; i < gathers_per_group; i += 8) {
@@ -405,7 +342,7 @@ gather_peak_kernel(const float* __restrict__ table, uint32_t rows, uint32_t row_
     for (int u = 0; u < 8; ++u) {
       state = state * 1664525u + 1013904223u;            // LCG: the lanes of a group draw the same ids
       const uint32_t id = uint32_t((uint64_t(state) * rows) >> 32);
-      v[u] = ld_row_f32x4(row_ptr(base, id, row_bytes), pol_keep);
+      v[u] = F32x4::unpack(F32x4::load(row_addr(base, id, row_bytes), pol_keep));
     }
 #pragma unroll
     for (int u = 0; u < 8; ++u) { acc.x += v[u].x; acc.y += v[u].y; acc.z += v[u].z; acc.w += v[u].w; }
@@ -419,22 +356,17 @@ static void dispatch_aggregate(int wkind, bool div, cudaStream_t st, const WorkL
                                float* out, int64_t ldo, int f, int epi) {
   using T = typename P::T;
   constexpr int kWin = LANES * P::kPer * V;
-#define GTA_AGG(K, D)                                                                                               \
-  do {                                                                                                              \
-    auto kern = aggregate_kernel<P, V, LANES, K, D>;                                                                \
-    dim3 grid = persistent_grid(kern, wl, LANES, 1, ex);                                                  \
-    grid.y = (unsigned)((f + kWin - 1) / kWin);                                                                     \
-    kern<<<grid, kAggThreads, 0, st>>>(with_take(wl, take_for(kern, wl, LANES)), ex, w, wh, rowden, x,    \
-                                       uint32_t(ldx * sizeof(T)), out, ldo, f, epi);                                \
-  } while (0)
-  if (wkind == 0) GTA_AGG(0, false);
-  else if (wkind == 1 && !div) GTA_AGG(1, false);
-  else if (wkind == 1 && div) GTA_AGG(1, true);
+  const int grid_y = (f + kWin - 1) / kWin;
+  auto launch = [&](auto kernel) {
+    launch_persistent(kernel, wl, ex, LANES, grid_y, st, w, wh, rowden, x, uint32_t(ldx * sizeof(T)), out, ldo, f, epi);
+  };
+  if (wkind == 0) launch(aggregate_kernel<P, V, LANES, 0, false>);
+  else if (wkind == 1 && !div) launch(aggregate_kernel<P, V, LANES, 1, false>);
+  else if (wkind == 1 && div) launch(aggregate_kernel<P, V, LANES, 1, true>);
   else if constexpr (V == 1) {
-    if (!div) GTA_AGG(2, false);
-    else GTA_AGG(2, true);
+    if (!div) launch(aggregate_kernel<P, V, LANES, 2, false>);
+    else launch(aggregate_kernel<P, V, LANES, 2, true>);
   }
-#undef GTA_AGG
 }
 
 // ---- the two aggregation entry points, for either storage type of the gathered table ---------------
@@ -471,11 +403,11 @@ static int aggregate_impl(const char* who, const int32_t* items_, int64_t num_it
   constexpr int kRow = 16 / int(sizeof(T));          // elements per 16 bytes: the row pitch granule
   cudaStream_t st = static_cast<cudaStream_t>(stream_);
   GTA_REQUIRE(f > 0 && f % 4 == 0, "%s: f=%d must be a positive multiple of 4 (pad the table)", who, f);
-  GTA_REQUIRE(num_items >= 0 && num_items < (int64_t(1) << 31) - 64, "%s: bad item count", who);
-  WorkList wl{reinterpret_cast<const int4*>(items_), num_items, row_slots, num_slots, indices, partials, nullptr, nullptr, 1, 0, 0};
-  int rc = prepare_worklist(who, wl, chain_state, f, phases, st);
-  if (rc != GTA_OK) return rc;
-  if (num_items == 0 || !(phases & GTA_PHASE_MAIN)) return GTA_OK;
+  WorkList wl;
+  bool launch = false;
+  int rc = prepare_worklist(who, items_, num_items, row_slots, num_slots, indices, partials, chain_state, f, phases, st,
+                            &wl, &launch);
+  if (rc != GTA_OK || !launch) return rc;
   GTA_REQUIRE(items_ && indices && x && out, "%s: null pointer", who);
   GTA_REQUIRE(ldx % kRow == 0 && ldo % 4 == 0 && ldx >= f && ldo >= f && ldx * int64_t(sizeof(T)) < (int64_t(1) << 32),
               "%s: leading dimensions must be whole 16-byte pieces, >= f, and a row below 4 GiB", who);
@@ -537,11 +469,11 @@ int gta_aggregate_edge_sum_f32(const int32_t* items_, int64_t num_items, const i
   const char* who = "gta_aggregate_edge_sum_f32";
   cudaStream_t st = static_cast<cudaStream_t>(stream_);
   GTA_REQUIRE(f > 0 && f % 4 == 0, "%s: f=%d must be a positive multiple of 4 (pad the table)", who, f);
-  GTA_REQUIRE(num_items >= 0 && num_items < (int64_t(1) << 31) - 64, "%s: bad item count", who);
-  WorkList wl{reinterpret_cast<const int4*>(items_), num_items, row_slots, num_slots, indices, partials, nullptr, nullptr, 1, 0, 0};
-  int rc = prepare_worklist(who, wl, chain_state, f, phases, st);
-  if (rc != GTA_OK) return rc;
-  if (num_items == 0 || !(phases & GTA_PHASE_MAIN)) return GTA_OK;
+  WorkList wl;
+  bool launch = false;
+  int rc = prepare_worklist(who, items_, num_items, row_slots, num_slots, indices, partials, chain_state, f, phases, st,
+                            &wl, &launch);
+  if (rc != GTA_OK || !launch) return rc;
   GTA_REQUIRE(items_ && out && (edge || x || rowterm), "%s: null pointer (at least one of edge / x / rowterm is needed)", who);
   GTA_REQUIRE(!x || indices, "%s: indices are required to gather x", who);
   GTA_REQUIRE(unary >= GTA_UN_EXP_LEAKY_RELU && unary <= GTA_UN_COPY, "%s: bad unary %d", who, unary);
@@ -554,29 +486,24 @@ int gta_aggregate_edge_sum_f32(const int32_t* items_, int64_t num_items, const i
               "%s: rowterm must be 16-byte aligned rows >= f", who);
   Exchange ex;
   memset(&ex, 0, sizeof(ex));
-#define GTA_ES2(L, HX, HE)                                                                                          \
-  do {                                                                                                              \
-    auto kern = edge_sum_kernel<L, HX, HE>;                                                                         \
-    dim3 grid = persistent_grid(kern, wl, L, 1, ex);                                                                \
-    grid.y = (unsigned)((f + 127) / 128);                                                                           \
-    kern<<<grid, kAggThreads, 0, st>>>(with_take(wl, take_for(kern, wl, L)), ex, edge, lde, x, uint32_t(ldx * 4),   \
-                                       rowterm, ldr, unary, slope, out, ldo, f, epilogue);                          \
-  } while (0)
-#define GTA_ES(L)                                                                                                   \
-  do {                                                                                                              \
-    if (x && edge) GTA_ES2(L, true, true);                                                                          \
-    else if (x) GTA_ES2(L, true, false);                                                                            \
-    else if (edge) GTA_ES2(L, false, true);                                                                         \
-    else GTA_ES2(L, false, false);                                                                                  \
-  } while (0)
-  switch (lanes_for(f, 4)) {
-    case 4: GTA_ES(4); break;
-    case 8: GTA_ES(8); break;
-    case 16: GTA_ES(16); break;
-    default: GTA_ES(32); break;
+  const int lanes = lanes_for(f, 4);
+  auto launch_es = [&](auto kernel) {
+    launch_persistent(kernel, wl, ex, lanes, (f + 127) / 128, st, edge, lde, x, uint32_t(ldx * 4), rowterm, ldr, unary,
+                      slope, out, ldo, f, epilogue);
+  };
+  auto for_terms = [&](auto lanes_c) {
+    constexpr int L = decltype(lanes_c)::value;
+    if (x && edge) launch_es(edge_sum_kernel<L, true, true>);
+    else if (x) launch_es(edge_sum_kernel<L, true, false>);
+    else if (edge) launch_es(edge_sum_kernel<L, false, true>);
+    else launch_es(edge_sum_kernel<L, false, false>);
+  };
+  switch (lanes) {
+    case 4: for_terms(std::integral_constant<int, 4>()); break;
+    case 8: for_terms(std::integral_constant<int, 8>()); break;
+    case 16: for_terms(std::integral_constant<int, 16>()); break;
+    default: for_terms(std::integral_constant<int, 32>()); break;
   }
-#undef GTA_ES
-#undef GTA_ES2
   GTA_CHECK_LAUNCH("edge_sum_kernel");
   return GTA_OK;
 }

@@ -5,6 +5,8 @@
 #include <cuda_bf16.h>
 #include <string.h>
 
+#include <type_traits>
+
 #include "common.cuh"
 #include "exchange.cuh"
 
@@ -35,18 +37,6 @@ namespace gta {
 #endif
 #ifndef GTA_LLH_UNROLL
 #define GTA_LLH_UNROLL 8
-#endif
-#ifndef GTA_AGG_FASTEXP
-#define GTA_AGG_FASTEXP 1
-#endif
-#ifndef GTA_GAT_FORCE_LLH
-#define GTA_GAT_FORCE_LLH 0       // experiment: run the lane-local-head kernel for every head count
-#endif
-#ifndef GTA_ITEM_PREFETCH
-#define GTA_ITEM_PREFETCH 1       // stage the NEXT item's record and first ids / el while the current one is folded
-#endif
-#ifndef GTA_PUBLISH_FENCE
-#define GTA_PUBLISH_FENCE 0       // 1: an extra fence.sc in front of the release store of a chain publish (round-2 form)
 #endif
 constexpr int kAggThreads = GTA_AGG_THREADS;
 constexpr int kAggWarps = kAggThreads / 32;
@@ -81,9 +71,6 @@ __device__ __forceinline__ void chain_publish(int32_t* flag) {
   // st.release is cumulative over what the barrier ordered before this lane (the idiom of CUTLASS's Semaphore::release:
   // barrier, then one thread's st.release.gpu); a __threadfence() in front of it is a second, sequentially consistent
   // fence (membar.gl) per item and buys nothing
-#if GTA_PUBLISH_FENCE
-  __threadfence();
-#endif
   asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(flag), "r"(1) : "memory");
 }
 // predecessor state was written by another SM during this launch: read it at L2, never from L1
@@ -109,26 +96,33 @@ __device__ __forceinline__ void for_groups_in_order(int lane, bool chained, F&& 
     }
   }
 }
-
-// ---- the next item, staged while the current one runs ------------------------------------------
-// An item costs a chain of dependent loads before its first gather can issue: the item record, then its first source
-// ids (streamed from DRAM) and el row, then the er rows of those ids; and two row_slots reads in front of the chain fold.
-// Measured on the Reddit shape (agg_probe, items of 20 edges against items of 164): about 5 us of warp time per item
-// whatever its length, a quarter of the kernel.  The record of the NEXT item and the slot range of the CURRENT row are
-// therefore copied into shared memory asynchronously at the top of an item (no registers held across the gather loop),
-// and the next item's el row and first two id batches are requested right after the gather loop, so that they travel
-// while the chain fold of the current item waits for its predecessor.
-struct NextItem {
-  int4 item;
-  int32_t s0, s1, pad0, pad1;
-};
-__device__ __forceinline__ void cp_async_16(void* smem, const void* gmem) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(uint32_t(__cvta_generic_to_shared(smem))), "l"(gmem) : "memory");
+// The end of item `it` (record {row, first edge, count, slot}; slot < 0: the row has no other item).  A chained item
+// that is not the first of its row waits for its predecessor's flag and calls fold(it.w - 1) to merge that slot's
+// state; then it either calls save(it.w) and publishes, or -- last item of the row, or not chained -- calls finish()
+// to write the output.  slots() returns the row's slot range {first, end} and is only called for a chained item.
+template <int LANES, typename Slots, typename Fold, typename Save, typename Finish>
+__device__ __forceinline__ void chain_step(int32_t* flags, int lane, const int4& it, bool chained, Slots&& slots,
+                                           Fold&& fold, Save&& save, Finish&& finish) {
+  for_groups_in_order<LANES>(lane, chained, [&]() {
+    const bool leader = (lane & (LANES - 1)) == 0;
+    bool last = true;
+    if (chained) {
+      const int2 s = slots();
+      last = it.w == s.y - 1;
+      if (it.w != s.x) {
+        if (leader) chain_wait(flags + it.w - 1);
+        __syncwarp(group_mask<LANES>(lane));
+        fold(it.w - 1);
+      }
+      if (!last) {
+        save(it.w);
+        __syncwarp(group_mask<LANES>(lane));          // the group's stores happen-before lane 0's release
+        if (leader) chain_publish(flags + it.w);
+      }
+    }
+    if (last) finish();
+  });
 }
-__device__ __forceinline__ void cp_async_4(void* smem, const void* gmem) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(uint32_t(__cvta_generic_to_shared(smem))), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
 template <int LANES>
 __device__ __forceinline__ float group_max(float v) {
@@ -147,53 +141,9 @@ __device__ __forceinline__ int warp_max_i32(int v) {
   for (int o = 16; o > 0; o >>= 1) v = max(v, __shfl_xor_sync(0xffffffffu, v, o));
   return v;
 }
-// gathered feature row, 128 bits per lane.  GTA_AGG_GATHER picks the cache policy (measured on B200,
-// see DESIGN.md): 0 = L1 no-allocate, 1 = default, 2 = L1 no-allocate + L2 evict_last, 3 = L2 evict_last,
-// 4 = as 2 without .nc (coherent path)
-#ifndef GTA_AGG_GATHER
-#define GTA_AGG_GATHER 4
-#endif
-__device__ __forceinline__ float4 ld_row_f32x4(const float* p, uint64_t pol_keep) {
-  float4 v;
-#if GTA_AGG_GATHER == 0
-  asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];"
-               : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
-#elif GTA_AGG_GATHER == 1
-  asm volatile("ld.global.nc.v4.f32 {%0,%1,%2,%3}, [%4];"
-               : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
-#elif GTA_AGG_GATHER == 2
-  asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.f32 {%0,%1,%2,%3}, [%4], %5;"
-               : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p), "l"(pol_keep));
-#elif GTA_AGG_GATHER == 3
-  asm volatile("ld.global.nc.L2::cache_hint.v4.f32 {%0,%1,%2,%3}, [%4], %5;"
-               : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p), "l"(pol_keep));
-#else      // 4: as 2 but through the coherent path (no .nc)
-  asm volatile("ld.global.L1::no_allocate.L2::cache_hint.v4.f32 {%0,%1,%2,%3}, [%4], %5;"
-               : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p), "l"(pol_keep));
-#endif
-  return v;
-}
-// address of a gathered row: base + id * row_bytes.  Written as a 64-bit multiply-add of two 32-bit
-// values so ptxas emits ONE IMAD.WIDE.U32 with the lane's base pointer as the addend (the round-1 inline
-// mad.wide.u32 was split into IMAD.WIDE + IADD3 + IADD3.X once the base pair was not register-aligned).
-__device__ __forceinline__ const float* row_ptr(const float* base, uint32_t id, uint32_t row_bytes) {
-  return reinterpret_cast<const float*>(reinterpret_cast<const char*>(base) + uint64_t(id) * row_bytes);
-}
-// exp of a non-positive softmax exponent.  GTA_AGG_FASTEXP=1: ex2.approx path (relative error about
-// 2e-7 + |x| 1e-7; terms that matter have small |x|), two instructions instead of about ten.
-__device__ __forceinline__ float softmax_exp(float x) {
-#if GTA_AGG_FASTEXP
-  return __expf(x);
-#else
-  return expf(x);
-#endif
-}
-__device__ __forceinline__ void fma4(float4& acc, float w, const float4& v) {
-  acc.x = fmaf(w, v.x, acc.x);
-  acc.y = fmaf(w, v.y, acc.y);
-  acc.z = fmaf(w, v.z, acc.z);
-  acc.w = fmaf(w, v.w, acc.w);
-}
+// exp of a non-positive softmax exponent: the ex2.approx path (relative error about 2e-7 + |x| 1e-7; terms that matter
+// have small |x|), two instructions instead of about ten
+__device__ __forceinline__ float softmax_exp(float x) { return __expf(x); }
 __device__ __forceinline__ float4 epilogue4(float4 a, float scale, int epi) {
   a.x = apply_epilogue(a.x * scale, epi);
   a.y = apply_epilogue(a.y * scale, epi);
@@ -266,6 +216,74 @@ __device__ __forceinline__ void cursor_next(ItemCursor& c, const WorkList& wl, i
   }
 }
 
+// ---- the next item, staged while the current one runs ------------------------------------------
+// An item costs a chain of dependent loads before its first gather can issue: the item record, then its first source
+// ids (streamed from DRAM) and el row, then the er rows of those ids; and two row_slots reads in front of the chain fold.
+// Measured on the Reddit shape (agg_probe, items of 20 edges against items of 164): about 5 us of warp time per item
+// whatever its length, a quarter of the kernel.  The record of the NEXT item and the slot range of the CURRENT row are
+// therefore copied into shared memory asynchronously at the top of an item (no registers held across the gather loop),
+// and the next item's el row and first two id batches are requested right after the gather loop, so that they travel
+// while the chain fold of the current item waits for its predecessor.
+struct NextItem {
+  int4 item;
+  int32_t s0, s1, pad0, pad1;
+};
+__device__ __forceinline__ void cp_async_16(void* smem, const void* gmem) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(uint32_t(__cvta_generic_to_shared(smem))), "l"(gmem) : "memory");
+}
+__device__ __forceinline__ void cp_async_4(void* smem, const void* gmem) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(uint32_t(__cvta_generic_to_shared(smem))), "l"(gmem) : "memory");
+}
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
+
+// A warp group's walk of the work list with that staging, from the cursor of its first group-step (whose item is read
+// directly).  Per item, in this order:
+//   claim()        top of the item: take the next group-step, cp.async its record and this row's slot range
+//   land()         after the gather loop: wait for the copies, return the next record and read `slots` (the
+//                  staging entry is free again)
+//   advance(next)  after the chain step: the next item becomes the current one
+// The kernel requests its own inputs of `it` after construction and of the next item right after land().
+template <int LANES>
+struct ItemStage {
+  ItemCursor cur, nxt;
+  int4 it = make_int4(0, 0, 0, -1);
+  bool have = false, next_have;
+  int2 slots;                // this row's slot range, read in land() when the item is chained
+  NextItem* nx;
+  __device__ __forceinline__ ItemStage(const WorkList& wl, const ItemCursor& first, int lane, NextItem* entry)
+      : cur(first), nx(entry) {
+    const int64_t group = int64_t(cur.first) + lane / LANES;
+    have = group < wl.num_items;
+    if (have) it = __ldg(wl.items + group);
+  }
+  __device__ __forceinline__ void claim(const WorkList& wl, int32_t* counter, int lane) {
+    nxt = cur;
+    cursor_next<LANES>(nxt, wl, counter, lane);
+    const int64_t ngroup = int64_t(nxt.first) + lane / LANES;
+    next_have = nxt.first < wl.num_items && ngroup < wl.num_items;
+    if ((lane & (LANES - 1)) == 0) {
+      if (next_have) cp_async_16(&nx->item, wl.items + ngroup);
+      if (have && it.w >= 0) {
+        cp_async_4(&nx->s0, wl.row_slots + it.x);
+        cp_async_4(&nx->s1, wl.row_slots + it.x + 1);
+      }
+    }
+  }
+  __device__ __forceinline__ int4 land(bool chained) {
+    cp_async_wait_all();
+    __syncwarp();
+    const int4 next = next_have ? nx->item : make_int4(0, 0, 0, -1);
+    slots = make_int2(chained ? nx->s0 : 0, chained ? nx->s1 : 0);
+    __syncwarp();          // everybody has read the staging entry before lane 0 of the group overwrites it
+    return next;
+  }
+  __device__ __forceinline__ void advance(const int4& next) {
+    cur = nxt;
+    it = next;
+    have = next_have;
+  }
+};
+
 // ----------------------------------------------------------------------------------------
 // storage type of the gathered table: fp32, or bf16 with fp32 accumulation (SURVEY.md section 8d "bf16 mode";
 // the reference's IR declares data_format FP16, template/IR_defination.yaml:10-27).  A lane always moves
@@ -290,6 +308,9 @@ struct F32x4 {
   static __device__ __forceinline__ Raw zero() { return make_uint4(0u, 0u, 0u, 0u); }
   static __device__ __forceinline__ void unpack(const Raw& r, float (&f)[4]) {
     f[0] = __uint_as_float(r.x); f[1] = __uint_as_float(r.y); f[2] = __uint_as_float(r.z); f[3] = __uint_as_float(r.w);
+  }
+  static __device__ __forceinline__ float4 unpack(const Raw& r) {
+    return make_float4(__uint_as_float(r.x), __uint_as_float(r.y), __uint_as_float(r.z), __uint_as_float(r.w));
   }
 };
 struct Bf16x8 {
@@ -321,6 +342,9 @@ struct Bf16x4 {
     f[2] = __uint_as_float(r.y << 16); f[3] = __uint_as_float(r.y & 0xffff0000u);
   }
 };
+// address of a gathered row: base + id * row_bytes.  Written as a 64-bit multiply-add of two 32-bit
+// values so ptxas emits ONE IMAD.WIDE.U32 with the lane's base pointer as the addend (an inline
+// mad.wide.u32 was split into IMAD.WIDE + IADD3 + IADD3.X once the base pair was not register-aligned).
 __device__ __forceinline__ const char* row_addr(const char* base, uint32_t id, uint32_t row_bytes) {
   return base + uint64_t(id) * row_bytes;
 }
@@ -359,7 +383,7 @@ constexpr int kGatUnroll = GTA_GAT_UNROLL;
 constexpr int kLlhUnroll = GTA_LLH_UNROLL;
 
 // ----------------------------------------------------------------------------------------
-// host side: lanes per item, persistent grid, exchange descriptor, work-list preparation
+// host side: lanes per item, persistent launch, exchange descriptor, work-list preparation
 // ----------------------------------------------------------------------------------------
 // lanes per item for rows of f features, kper features per 16-byte piece, v pieces per lane
 static int lanes_for(int f, int kper = 4, int v = 1) {
@@ -390,21 +414,20 @@ static int32_t take_for(K kernel, const WorkList& wl, int lanes) {
   return (wl.take == 0 && wl.num_items / (warps * groups) >= 32) ? 0 : 1;      // wl.take == 0: the caller's hint
 }
 
-template <typename K>
-static dim3 persistent_grid(K kernel, const WorkList& wl, int lanes, int f, const Exchange& ex) {
-  const int64_t num_items = wl.num_items;
-  const int64_t need = (num_items * lanes + kAggThreads - 1) / kAggThreads;
+// Persistent launch of an aggregation kernel whose parameters are (WorkList, Exchange, args...): as many CTAs as the
+// items need, at most as many as are resident, times grid_y feature windows, with the item fetch chosen for this list.
+template <typename K, typename... Args>
+static void launch_persistent(K kernel, WorkList wl, const Exchange& ex, int lanes, int grid_y, cudaStream_t st,
+                              Args... args) {
+  wl.take = take_for(kernel, wl, lanes);
+  const int64_t need = (wl.num_items * lanes + kAggThreads - 1) / kAggThreads;
   int64_t cap = resident_ctas(kernel);
   // the copy CTAs of an exchange come first in the grid, so they are resident before any CTA can wait on them;
   // with static striding every work CTA must be resident too (a chain may wait on any of them)
   const int64_t copy = ex.world > 1 ? ex.copy_ctas : 0;
-  if (take_for(kernel, wl, lanes) == 0 && cap > copy + 1) cap -= copy;
-  return dim3((unsigned)((need < cap ? need : cap) + copy), (unsigned)((f + 127) / 128));
-}
-
-static WorkList with_take(WorkList wl, int32_t take) {
-  wl.take = take;
-  return wl;
+  if (wl.take == 0 && cap > copy + 1) cap -= copy;
+  const dim3 grid((unsigned)((need < cap ? need : cap) + copy), (unsigned)grid_y);
+  kernel<<<grid, kAggThreads, 0, st>>>(wl, ex, args...);
 }
 
 // gta_exchange_t (host) -> Exchange (kernel parameter); arrived[] lives behind the item counters
@@ -438,31 +461,42 @@ static int make_exchange(const char* who, const gta_exchange_t* h, int32_t* arri
   return GTA_OK;
 }
 
-// common argument checks, the RESET phase (clear the chain flags of every feature window) and the item
-// counters (cleared before every launch).  chain_state = [windows][num_slots] flags, then [windows] item
-// counters, then GTA_MAX_RANKS slot-arrival counters of an exchange.
-static int prepare_worklist(const char* who, WorkList& wl, int32_t* chain_state, int32_t f, int32_t phases,
-                            cudaStream_t st) {
+// The work list of an entry point: the common argument checks, the RESET phase (clear the chain flags of every
+// feature window) and the item counters (cleared before every launch).  chain_state = [windows][num_slots] flags,
+// then [windows] item counters, then GTA_MAX_RANKS slot-arrival counters of an exchange.  *launch: the call has a
+// MAIN phase with items to reduce.
+static int prepare_worklist(const char* who, const int32_t* items, int64_t num_items, const int32_t* row_slots,
+                            int64_t num_slots, const int32_t* indices, float* partials, int32_t* chain_state, int32_t f,
+                            int32_t phases, cudaStream_t st, WorkList* wl, bool* launch) {
+  *launch = false;
+  GTA_REQUIRE(num_items >= 0 && num_items < (int64_t(1) << 31) - 64, "%s: bad item count", who);
   GTA_REQUIRE(chain_state, "%s: chain_state is required (chain flags and the item counters live there)", who);
-  GTA_REQUIRE(wl.num_slots == 0 || (wl.partials && wl.row_slots),
-              "%s: partials and row_slots are required for %lld slots", who, (long long)wl.num_slots);
+  GTA_REQUIRE(num_slots == 0 || (partials && row_slots),
+              "%s: partials and row_slots are required for %lld slots", who, (long long)num_slots);
   const size_t windows = size_t((f + 127) / 128);
-  wl.chain_flags = chain_state;
-  wl.work_counter = chain_state + windows * size_t(wl.num_slots);
-  if ((phases & GTA_PHASE_RESET) && wl.num_slots > 0) {
-    GTA_CUDA(cudaMemsetAsync(wl.chain_flags, 0, windows * size_t(wl.num_slots) * sizeof(int32_t), st));
+  *wl = WorkList{};
+  wl->items = reinterpret_cast<const int4*>(items);
+  wl->num_items = num_items;
+  wl->row_slots = row_slots;
+  wl->num_slots = num_slots;
+  wl->indices = indices;
+  wl->partials = partials;
+  wl->chain_flags = chain_state;
+  wl->work_counter = chain_state + windows * size_t(num_slots);
+  wl->take = (phases & GTA_PHASE_STATIC) ? 0 : 1;
+  if ((phases & GTA_PHASE_RESET) && num_slots > 0) {
+    GTA_CUDA(cudaMemsetAsync(wl->chain_flags, 0, windows * size_t(num_slots) * sizeof(int32_t), st));
     count_launch();
   }
-  wl.take = (phases & GTA_PHASE_STATIC) ? 0 : 1;
-  if ((phases & GTA_PHASE_MAIN) && wl.num_items > 0) {
-    GTA_CUDA(cudaMemsetAsync(wl.work_counter, 0, (windows + GTA_MAX_RANKS) * sizeof(int32_t), st));
-    count_launch();
-    CachePolicies pol;
-    int rc = cache_policies(&pol);
-    if (rc != GTA_OK) return rc;
-    wl.pol_stream = pol.stream;
-    wl.pol_keep = pol.keep;
-  }
+  if (!(phases & GTA_PHASE_MAIN) || num_items == 0) return GTA_OK;
+  GTA_CUDA(cudaMemsetAsync(wl->work_counter, 0, (windows + GTA_MAX_RANKS) * sizeof(int32_t), st));
+  count_launch();
+  CachePolicies pol;
+  const int rc = cache_policies(&pol);
+  if (rc != GTA_OK) return rc;
+  wl->pol_stream = pol.stream;
+  wl->pol_keep = pol.keep;
+  *launch = true;
   return GTA_OK;
 }
 

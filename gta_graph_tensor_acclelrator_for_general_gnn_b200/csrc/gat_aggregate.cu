@@ -126,9 +126,7 @@ gat_aggregate_kernel(const WorkList wl, const Exchange ex, const float* __restri
   constexpr int kWindow = LANES * KP;
   __shared__ __align__(16) uint2 s_e[kAggWarps][H * kS];
   __shared__ BoundCache<H> s_bound[kAggWarps][32 / LANES];
-#if GTA_ITEM_PREFETCH
   __shared__ __align__(16) NextItem s_next[kAggWarps][32 / LANES];
-#endif
   if (ex.world > 1 && blockIdx.y == 0 && blockIdx.x < ex.copy_ctas) {
     exchange_pull(ex, blockIdx.x);          // these CTAs move the peers' slots; everybody else reduces
     return;
@@ -152,12 +150,10 @@ gat_aggregate_kernel(const WorkList wl, const Exchange ex, const float* __restri
   const int stats = f + int(blockIdx.y) * gat_stats_stride(H);
   const char* zf = reinterpret_cast<const char*>(z + (fo < f ? fo : 0));
 
-  ItemCursor cur = cursor_begin<LANES>(wl, ex, counter, lane);
+  const ItemCursor first = cursor_begin<LANES>(wl, ex, counter, lane);
   int32_t landed = 0;          // exchange_gate: highest peer slot this lane has seen complete
   // what an item needs before its first batch: the record, the row's el, the ids of its first two batches and its
   // last id (sources ascend: the last id names the highest slot / statistics block the item touches)
-  int4 it = make_int4(0, 0, 0, -1);
-  bool have = false;
   float elr[H];
   int idx_cur = 0, idx_nxt = 0, last_src = 0;
   const bool want_last = ex.world > 1 || er_stats != nullptr;
@@ -173,37 +169,13 @@ gat_aggregate_kernel(const WorkList wl, const Exchange ex, const float* __restri
     if (LANES + l < cnt) idx_nxt = ld_stream_i32(ib + LANES + l, pol_stream);
     last_src = (cnt > 0 && want_last) ? __ldg(ib + cnt - 1) : 0;
   };
-#if GTA_ITEM_PREFETCH
-  NextItem* nx = &s_next[threadIdx.x >> 5][lane / LANES];
-  {
-    const int64_t group = int64_t(cur.first) + lane / LANES;
-    have = group < wl.num_items;
-    if (have) it = __ldg(wl.items + group);
-    request_inputs(it, have);
-  }
-#endif
-  while (cur.first < wl.num_items) {
-#if GTA_ITEM_PREFETCH
+  ItemStage<LANES> stage(wl, first, lane, &s_next[threadIdx.x >> 5][lane / LANES]);
+  request_inputs(stage.it, stage.have);
+  while (stage.cur.first < wl.num_items) {
     // claim the next item now and let its record (and this row's slot range) travel into shared memory under the gathers
-    ItemCursor nxt = cur;
-    cursor_next<LANES>(nxt, wl, counter, lane);
-    const int64_t ngroup = int64_t(nxt.first) + lane / LANES;
-    const bool nhave = nxt.first < wl.num_items && ngroup < wl.num_items;
-    if (l == 0) {
-      if (nhave) cp_async_16(&nx->item, wl.items + ngroup);
-      if (have && it.w >= 0) {
-        cp_async_4(&nx->s0, wl.row_slots + it.x);
-        cp_async_4(&nx->s1, wl.row_slots + it.x + 1);
-      }
-    }
-#else
-    {
-      const int64_t group = int64_t(cur.first) + lane / LANES;
-      have = group < wl.num_items;
-      it = have ? __ldg(wl.items + group) : make_int4(0, 0, 0, -1);
-      request_inputs(it, have);
-    }
-#endif
+    stage.claim(wl, counter, lane);
+    const int4 it = stage.it;
+    const bool have = stage.have;
     const bool active = have && fo < f;
     const int count = have ? it.z : 0;
     const int max_count = (LANES == 32) ? count : warp_max_i32(count);
@@ -330,30 +302,14 @@ gat_aggregate_kernel(const WorkList wl, const Exchange ex, const float* __restri
 #pragma unroll
     for (int h = 0; h < H; ++h) s[h] = group_sum<LANES>(s[h]);
     const bool chained = have && it.w >= 0;
-#if GTA_ITEM_PREFETCH
     // the gather loop is over: elr / idx_* are free, the staged record has long arrived.  Request the next item's
     // inputs now; they travel while this item's chain fold waits for its predecessor and writes its state.
-    cp_async_wait_all();
-    __syncwarp();
-    const int4 itn = nhave ? nx->item : make_int4(0, 0, 0, -1);
-    const int slot0 = chained ? nx->s0 : 0, slot1 = chained ? nx->s1 : 0;
-    __syncwarp();          // everybody has read the staging entry before lane 0 of the group overwrites it
-    request_inputs(itn, nhave);
-#endif
-    for_groups_in_order<LANES>(lane, chained, [&]() {
-      bool last = true;
-      if (chained) {
-#if GTA_ITEM_PREFETCH
-        const int s0 = slot0, s1 = slot1;
-#else
-        const int s0 = __ldg(wl.row_slots + it.x), s1 = __ldg(wl.row_slots + it.x + 1);
-#endif
-        last = it.w == s1 - 1;
-        if (it.w != s0) {
+    const int4 next = stage.land(chained);
+    request_inputs(next, stage.next_have);
+    chain_step<LANES>(flags, lane, it, chained, [&]() { return stage.slots; },
+        [&](int prev_slot) {
           // fold the state of slots [s0, it.w) in: (max, sum, acc) triples merge like the online softmax itself
-          if (l == 0) chain_wait(flags + it.w - 1);
-          __syncwarp(group_mask<LANES>(lane));
-          const float* prev = wl.partials + int64_t(it.w - 1) * pstride;
+          const float* prev = wl.partials + int64_t(prev_slot) * pstride;
           float a_mine = 1.f, b_mine = 1.f;
 #pragma unroll
           for (int h = 0; h < H; ++h) {
@@ -374,37 +330,28 @@ gat_aggregate_kernel(const WorkList wl, const Exchange ex, const float* __restri
 #pragma unroll
             for (int c = 0; c < KP; ++c) acc[c] = fmaf(p[c], a_mine, acc[c] * b_mine);
           }
-        }
-        if (!last) {
-          float* part = wl.partials + int64_t(it.w) * pstride;
+        },
+        [&](int slot) {
+          float* part = wl.partials + int64_t(slot) * pstride;
           if (active) st_state<KP>(part + fo, acc);
           if (l < H) {
             part[stats + l] = pick<H>(m, l);
             part[stats + H + l] = pick<H>(s, l);
           }
-          __syncwarp(group_mask<LANES>(lane));          // the group's stores happen-before lane 0's release
-          if (l == 0) chain_publish(flags + it.w);
-        }
-      }
-      if (last && have) {
-        if (active) {
-          const float sh = pick<H>(s, head);
-          st_out<KP>(out + int64_t(it.x) * ldo + fo, acc, sh > 0.f ? 1.f / sh : 0.f, epilogue);
-        }
-        if (blockIdx.y == 0 && l < H) {
-          const float ml = pick<H>(m, l);
-          if (rowmax) rowmax[int64_t(it.x) * H + l] = (count > 0 || it.w >= 0) && ml != -INFINITY ? ml : 0.f;
-          if (rowsum) rowsum[int64_t(it.x) * H + l] = pick<H>(s, l);
-        }
-      }
-    });
-#if GTA_ITEM_PREFETCH
-    cur = nxt;
-    it = itn;
-    have = nhave;
-#else
-    cursor_next<LANES>(cur, wl, counter, lane);
-#endif
+        },
+        [&]() {
+          if (!have) return;
+          if (active) {
+            const float sh = pick<H>(s, head);
+            st_out<KP>(out + int64_t(it.x) * ldo + fo, acc, sh > 0.f ? 1.f / sh : 0.f, epilogue);
+          }
+          if (blockIdx.y == 0 && l < H) {
+            const float ml = pick<H>(m, l);
+            if (rowmax) rowmax[int64_t(it.x) * H + l] = (count > 0 || it.w >= 0) && ml != -INFINITY ? ml : 0.f;
+            if (rowsum) rowsum[int64_t(it.x) * H + l] = pick<H>(s, l);
+          }
+        });
+    stage.advance(next);
   }
 }
 
@@ -458,7 +405,7 @@ gat_aggregate_llh_kernel(const WorkList wl, const Exchange ex, const float* __re
   const int fo = blockIdx.y * 128 + 4 * l;
   const int d = f / heads;          // HPL == 1: a multiple of 4;  HPL == 2: 2;  HPL == 4: 1
   const int head = (fo < f) ? fo / d : 0;          // the lane's first head (a multiple of HPL)
-  const float* erh = er + head;
+  const char* erh = reinterpret_cast<const char*>(er + head);
   const uint32_t er_bytes = uint32_t(lder) * 4u;
   uint32_t* sid = s_id[threadIdx.x >> 5];
   const uint32_t* mine = sid + (lane & ~(LANES - 1));
@@ -478,7 +425,7 @@ gat_aggregate_llh_kernel(const WorkList wl, const Exchange ex, const float* __re
     const int count = have ? it.z : 0;
     const int max_count = (LANES == 32) ? count : warp_max_i32(count);
     const int32_t* idx_base = wl.indices + it.y;
-    const float* zf = z + (active ? fo : 0);
+    const char* zf = reinterpret_cast<const char*>(z + (active ? fo : 0));
     float elh[HPL], m[HPL], s[HPL];
 #pragma unroll
     for (int k = 0; k < HPL; ++k) { elh[k] = 0.f; m[k] = -INFINITY; s[k] = 0.f; }
@@ -523,14 +470,14 @@ gat_aggregate_llh_kernel(const WorkList wl, const Exchange ex, const float* __re
           float erv[HPL];
 #pragma unroll
           for (int k = 0; k < HPL; ++k) erv[k] = 0.f;
-          if (ok) ldg_vec<HPL>(row_ptr(erh, id[u], er_bytes), erv);
+          if (ok) ldg_vec<HPL>(reinterpret_cast<const float*>(row_addr(erh, id[u], er_bytes)), erv);
 #pragma unroll
           for (int k = 0; k < HPL; ++k) e[u][k] = ok ? leaky(elh[k] + erv[k], slope) : -INFINITY;
         }
 #pragma unroll
         for (int u = 0; u < kU; ++u) {
           v[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (active && (j + u) < n) v[u] = ld_row_f32x4(row_ptr(zf, id[u], row_bytes), pol_keep);
+          if (active && (j + u) < n) v[u] = F32x4::unpack(F32x4::load(row_addr(zf, id[u], row_bytes), pol_keep));
         }
         if (!bounded) {
           // online softmax: new running maximum per head, rescale what has been accumulated.  A head that has
@@ -551,12 +498,11 @@ gat_aggregate_llh_kernel(const WorkList wl, const Exchange ex, const float* __re
         }
 #pragma unroll
         for (int u = 0; u < kU; ++u) {
-          // e = -inf for the padding of the last group: p = 0.  ex2.approx path: the argument is <= 0 and terms
-          // that matter have small |e - m|; relative error < 2e-6, inside the 1e-5 tolerance
+          // e = -inf for the padding of the last group: p = 0
           float p[HPL];
 #pragma unroll
           for (int k = 0; k < HPL; ++k) {
-            p[k] = (m[k] == -INFINITY) ? 0.f : __expf(e[u][k] - m[k]);
+            p[k] = (m[k] == -INFINITY) ? 0.f : softmax_exp(e[u][k] - m[k]);
             s[k] += p[k];
           }
           acc.x = fmaf(p[head_of<HPL>(0)], v[u].x, acc.x); acc.y = fmaf(p[head_of<HPL>(1)], v[u].y, acc.y);
@@ -568,16 +514,11 @@ gat_aggregate_llh_kernel(const WorkList wl, const Exchange ex, const float* __re
     // who publishes a head's statistics: the first lane of the head (width >= 4), or the one lane that owns it
     const bool head_leader = active && (HPL > 1 || (fo % d) == 0);
     const bool chained = have && it.w >= 0;
-    for_groups_in_order<LANES>(lane, chained, [&]() {
-      bool last = true;
-      if (chained) {
-        const int s0 = __ldg(wl.row_slots + it.x), s1 = __ldg(wl.row_slots + it.x + 1);
-        last = it.w == s1 - 1;
-        if (it.w != s0) {
-          if (l == 0) chain_wait(flags + it.w - 1);
-          __syncwarp(group_mask<LANES>(lane));
+    chain_step<LANES>(flags, lane, it, chained,
+        [&]() { return make_int2(__ldg(wl.row_slots + it.x), __ldg(wl.row_slots + it.x + 1)); },
+        [&](int prev_slot) {
           if (active) {
-            const float* prev = wl.partials + int64_t(it.w - 1) * pstride;
+            const float* prev = wl.partials + int64_t(prev_slot) * pstride;
             float a[HPL], b[HPL];
 #pragma unroll
             for (int k = 0; k < HPL; ++k) {
@@ -595,9 +536,9 @@ gat_aggregate_llh_kernel(const WorkList wl, const Exchange ex, const float* __re
             acc.z = fmaf(p.z, a[head_of<HPL>(2)], acc.z * b[head_of<HPL>(2)]);
             acc.w = fmaf(p.w, a[head_of<HPL>(3)], acc.w * b[head_of<HPL>(3)]);
           }
-        }
-        if (!last) {
-          float* part = wl.partials + int64_t(it.w) * pstride;
+        },
+        [&](int slot) {
+          float* part = wl.partials + int64_t(slot) * pstride;
           if (active) *reinterpret_cast<float4*>(part + fo) = acc;
           if (head_leader) {
 #pragma unroll
@@ -606,26 +547,23 @@ gat_aggregate_llh_kernel(const WorkList wl, const Exchange ex, const float* __re
               part[stats + heads + head + k] = s[k];
             }
           }
-          __syncwarp(group_mask<LANES>(lane));          // the group's stores happen-before lane 0's release
-          if (l == 0) chain_publish(flags + it.w);
-        }
-      }
-      if (last && active) {
-        float inv[HPL];
+        },
+        [&]() {
+          if (!active) return;
+          float inv[HPL];
 #pragma unroll
-        for (int k = 0; k < HPL; ++k) inv[k] = s[k] > 0.f ? 1.f / s[k] : 0.f;
-        st_stream_f32x4(out + int64_t(it.x) * ldo + fo,
-                        make_float4(apply_epilogue(acc.x * inv[head_of<HPL>(0)], epilogue), apply_epilogue(acc.y * inv[head_of<HPL>(1)], epilogue),
-                                    apply_epilogue(acc.z * inv[head_of<HPL>(2)], epilogue), apply_epilogue(acc.w * inv[head_of<HPL>(3)], epilogue)));
-        if (head_leader) {
+          for (int k = 0; k < HPL; ++k) inv[k] = s[k] > 0.f ? 1.f / s[k] : 0.f;
+          st_stream_f32x4(out + int64_t(it.x) * ldo + fo,
+                          make_float4(apply_epilogue(acc.x * inv[head_of<HPL>(0)], epilogue), apply_epilogue(acc.y * inv[head_of<HPL>(1)], epilogue),
+                                      apply_epilogue(acc.z * inv[head_of<HPL>(2)], epilogue), apply_epilogue(acc.w * inv[head_of<HPL>(3)], epilogue)));
+          if (head_leader) {
 #pragma unroll
-          for (int k = 0; k < HPL; ++k) {
-            if (rowmax) rowmax[int64_t(it.x) * heads + head + k] = (count > 0 || it.w >= 0) && m[k] != -INFINITY ? m[k] : 0.f;
-            if (rowsum) rowsum[int64_t(it.x) * heads + head + k] = s[k];
+            for (int k = 0; k < HPL; ++k) {
+              if (rowmax) rowmax[int64_t(it.x) * heads + head + k] = (count > 0 || it.w >= 0) && m[k] != -INFINITY ? m[k] : 0.f;
+              if (rowsum) rowsum[int64_t(it.x) * heads + head + k] = s[k];
+            }
           }
-        }
-      }
-    });
+        });
     cursor_next<LANES>(cur, wl, counter, lane);
   }
 }
@@ -707,23 +645,17 @@ static int dispatch_gat(int lanes, cudaStream_t st, const WorkList& wl, const Ex
                         const float* er, int64_t lder, float slope, const typename P::T* z, int64_t ldz, float* out, int64_t ldo,
                         int f, int epi, float* rowmax, float* rowsum, const uint32_t* er_stats, int stats_pitch,
                         int64_t col_block) {
-#define GTA_GAT(L)                                                                                                  \
-  do {                                                                                                              \
-    auto kern = gat_aggregate_kernel<P, L, H>;                                                                      \
-    dim3 grid = persistent_grid(kern, wl, L, 1, ex);                                                      \
-    grid.y = (unsigned)((f + L * P::kPer - 1) / (L * P::kPer));                                                     \
-    kern<<<grid, kAggThreads, 0, st>>>(with_take(wl, take_for(kern, wl, L)), ex, el, er, lder, slope, z,  \
-                                       uint32_t(ldz * sizeof(typename P::T)), out, ldo, f, epi, rowmax, rowsum,     \
-                                       er_stats,                                                                    \
-                                       stats_pitch, col_block);                                                     \
-  } while (0)
+  auto launch = [&](auto kernel, int lanes_c) {
+    launch_persistent(kernel, wl, ex, lanes_c, (f + lanes_c * P::kPer - 1) / (lanes_c * P::kPer), st, el, er, lder, slope, z,
+                      uint32_t(ldz * sizeof(typename P::T)), out, ldo, f, epi, rowmax, rowsum, er_stats, stats_pitch,
+                      col_block);
+  };
   switch (lanes) {
-    case 4: if (H <= 4) { GTA_GAT(4); return GTA_OK; } break;
-    case 8: if (H <= 8) { GTA_GAT(8); return GTA_OK; } break;
-    case 16: GTA_GAT(16); return GTA_OK;
-    case 32: GTA_GAT(32); return GTA_OK;
+    case 4: if (H <= 4) { launch(gat_aggregate_kernel<P, 4, H>, 4); return GTA_OK; } break;
+    case 8: if (H <= 8) { launch(gat_aggregate_kernel<P, 8, H>, 8); return GTA_OK; } break;
+    case 16: launch(gat_aggregate_kernel<P, 16, H>, 16); return GTA_OK;
+    case 32: launch(gat_aggregate_kernel<P, 32, H>, 32); return GTA_OK;
   }
-#undef GTA_GAT
   return GTA_ERR_UNSUPPORTED;
 }
 
@@ -760,11 +692,11 @@ static int gat_aggregate_impl(const char* who, const int32_t* items_, int64_t nu
   constexpr int kRow = 16 / int(sizeof(T));
   cudaStream_t st = static_cast<cudaStream_t>(stream_);
   GTA_REQUIRE(f > 0 && f % 4 == 0, "%s: f=%d must be a positive multiple of 4", who, f);
-  GTA_REQUIRE(num_items >= 0 && num_items < (int64_t(1) << 31) - 64, "%s: bad item count", who);
-  WorkList wl{reinterpret_cast<const int4*>(items_), num_items, row_slots, num_slots, indices, partials, nullptr, nullptr, 1, 0, 0};
-  int rc = prepare_worklist(who, wl, chain_state, f, phases, st);
-  if (rc != GTA_OK) return rc;
-  if (num_items == 0 || !(phases & GTA_PHASE_MAIN)) return GTA_OK;
+  WorkList wl;
+  bool launch = false;
+  int rc = prepare_worklist(who, items_, num_items, row_slots, num_slots, indices, partials, chain_state, f, phases, st,
+                            &wl, &launch);
+  if (rc != GTA_OK || !launch) return rc;
   GTA_REQUIRE(items_ && indices && el && er && z && out, "%s: null pointer", who);
   GTA_REQUIRE(ldz % kRow == 0 && ldo % 4 == 0 && ldz >= f && ldo >= f && ldz * int64_t(sizeof(T)) < (int64_t(1) << 32),
               "%s: leading dimensions must be whole 16-byte pieces, >= f, and a row below 4 GiB", who);
@@ -791,7 +723,7 @@ static int gat_aggregate_impl(const char* who, const int32_t* items_, int64_t nu
   // H <= 4 with whole pieces per head: staged kernel (all heads per lane, softmax once per 32-edge batch);  H >= 8, an
   // unusual H or heads narrower than a piece: lane-local-head kernel (per-head width a multiple of 4, or 2, or 1;
   // constant register footprint; fp32 tables only)
-  bool staged = !GTA_GAT_FORCE_LLH && (heads == 1 || heads == 2 || heads == 4);
+  bool staged = heads == 1 || heads == 2 || heads == 4;
   if constexpr (sizeof(T) == 4) staged = staged && (f / heads) % 4 == 0;
   if (staged) {
     if constexpr (sizeof(T) == 4) {
@@ -813,25 +745,22 @@ static int gat_aggregate_impl(const char* who, const int32_t* items_, int64_t nu
       return GTA_ERR_UNSUPPORTED;
     }
     const int lanes = lanes_for(f, 4);
-#define GTA_LLH2(L, HP)                                                                                                 \
-  gat_aggregate_llh_kernel<L, HP><<<persistent_grid(gat_aggregate_llh_kernel<L, HP>, wl, L, f, ex), kAggThreads, 0,      \
-                                    st>>>(with_take(wl, take_for(gat_aggregate_llh_kernel<L, HP>, wl, L)), ex, el, er,   \
-                                          lder, heads, slope, z, uint32_t(ldz) * 4u, out, ldo, f, epilogue, rowmax,      \
-                                          rowsum, er_stats, stats_pitch, col_block)
-#define GTA_LLH(L)                                                                                                      \
-  do {                                                                                                                  \
-    if (hpl == 1) GTA_LLH2(L, 1);                                                                                       \
-    else if (hpl == 2) GTA_LLH2(L, 2);                                                                                  \
-    else GTA_LLH2(L, 4);                                                                                                \
-  } while (0)
+    auto launch_llh = [&](auto kernel) {
+      launch_persistent(kernel, wl, ex, lanes, (f + 127) / 128, st, el, er, lder, heads, slope, z, uint32_t(ldz) * 4u, out,
+                        ldo, f, epilogue, rowmax, rowsum, er_stats, stats_pitch, col_block);
+    };
+    auto for_heads_per_lane = [&](auto lanes_c) {
+      constexpr int L = decltype(lanes_c)::value;
+      if (hpl == 1) launch_llh(gat_aggregate_llh_kernel<L, 1>);
+      else if (hpl == 2) launch_llh(gat_aggregate_llh_kernel<L, 2>);
+      else launch_llh(gat_aggregate_llh_kernel<L, 4>);
+    };
     switch (lanes) {
-      case 4: GTA_LLH(4); break;
-      case 8: GTA_LLH(8); break;
-      case 16: GTA_LLH(16); break;
-      default: GTA_LLH(32); break;
+      case 4: for_heads_per_lane(std::integral_constant<int, 4>()); break;
+      case 8: for_heads_per_lane(std::integral_constant<int, 8>()); break;
+      case 16: for_heads_per_lane(std::integral_constant<int, 16>()); break;
+      default: for_heads_per_lane(std::integral_constant<int, 32>()); break;
     }
-#undef GTA_LLH
-#undef GTA_LLH2
   } else {
     set_error("%s: %d heads on a bf16 table has no kernel yet (fp32 tables: any head count)", who, heads);
     return GTA_ERR_UNSUPPORTED;
