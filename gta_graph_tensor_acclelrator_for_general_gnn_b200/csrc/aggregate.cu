@@ -383,6 +383,8 @@ static int aggregate_run(const char* who, int wkind, bool div, cudaStream_t st, 
   // rows wider than one 32-lane pass of single pieces: two pieces per lane (one walk of the work list, not two)
   if (f > 32 * KP && wkind != 2) {
     dispatch_aggregate<P, 2, 32>(wkind, div, st, wl, ex, w, wh, rowden, x, ldx, out, ldo, f, epilogue);
+  } else if constexpr (KP == 8) {          // Bf16x8 only takes rows wider than 128 features: always 32 lanes
+    dispatch_aggregate<P, 1, 32>(wkind, div, st, wl, ex, w, wh, rowden, x, ldx, out, ldo, f, epilogue);
   } else {
     switch (lanes_for(f, KP)) {
       case 4: dispatch_aggregate<P, 1, 4>(wkind, div, st, wl, ex, w, wh, rowden, x, ldx, out, ldo, f, epilogue); break;
@@ -424,9 +426,11 @@ static int aggregate_impl(const char* who, const int32_t* items_, int64_t num_it
   rc = make_exchange(who, exchange, wl.work_counter + (f + 127) / 128, ldx * int64_t(sizeof(T)), &ex);
   if (rc != GTA_OK) return rc;
   GTA_REQUIRE(ex.world <= 1 || ex.table == reinterpret_cast<const char*>(x), "%s: x is not the exchange table", who);
+  // bf16: 16-byte pieces of 8 features for rows wider than 128 whose width (and per-head width) is whole pieces of 8;
+  // every other width of whole 4-feature pieces takes 8-byte pieces of 4 (two per lane above 128 features)
   if constexpr (sizeof(T) == 4) {
     rc = aggregate_run<F32x4>(who, wkind, div, st, wl, ex, w, wh, rowden, x, ldx, out, ldo, f, epilogue);
-  } else if (f <= 128) {
+  } else if (f <= 128 || f % 8 != 0 || (wkind == 2 && (f / wh) % 8 != 0)) {
     rc = aggregate_run<Bf16x4>(who, wkind, div, st, wl, ex, w, wh, rowden, x, ldx, out, ldo, f, epilogue);
   } else {
     rc = aggregate_run<Bf16x8>(who, wkind, div, st, wl, ex, w, wh, rowden, x, ldx, out, ldo, f, epilogue);

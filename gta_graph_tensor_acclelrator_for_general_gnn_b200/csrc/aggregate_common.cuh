@@ -291,10 +291,13 @@ struct ItemStage {
 // ----------------------------------------------------------------------------------------
 // A PIECE is what one lane moves of one gathered row: its storage type, how many features, how many bytes.
 //   F32x4   4 fp32 in 16 bytes            (512-byte rows at 32 lanes: the fp32 mode)
-//   Bf16x8  8 bf16 in 16 bytes            (rows wider than 128 features)
+//   Bf16x8  8 bf16 in 16 bytes            (rows wider than 128 features whose width, and per-head width, is a
+//                                          multiple of 8; always 32 lanes)
 //   Bf16x4  4 bf16 in  8 bytes            (rows of up to 128 features keep all 32 lanes on ONE item: the per-batch
 //                                          work -- staging, softmax -- is then spread over 32 edges, not 16; measured
-//                                          on the Reddit shape: Bf16x8 at 16 lanes per item was no faster than fp32)
+//                                          on the Reddit shape: Bf16x8 at 16 lanes per item was no faster than fp32.
+//                                          Also wider rows of any other multiple of 4: two pieces per lane in the
+//                                          aggregate, windows of 128 in the GAT kernel)
 struct F32x4 {
   using T = float;
   using Raw = uint4;

@@ -650,11 +650,15 @@ static int dispatch_gat(int lanes, cudaStream_t st, const WorkList& wl, const Ex
                       uint32_t(ldz * sizeof(typename P::T)), out, ldo, f, epi, rowmax, rowsum, er_stats, stats_pitch,
                       col_block);
   };
-  switch (lanes) {
-    case 4: if (H <= 4) { launch(gat_aggregate_kernel<P, 4, H>, 4); return GTA_OK; } break;
-    case 8: if (H <= 8) { launch(gat_aggregate_kernel<P, 8, H>, 8); return GTA_OK; } break;
-    case 16: launch(gat_aggregate_kernel<P, 16, H>, 16); return GTA_OK;
-    case 32: launch(gat_aggregate_kernel<P, 32, H>, 32); return GTA_OK;
+  if constexpr (P::kPer == 8) {          // Bf16x8 only takes rows wider than 128 features: always 32 lanes
+    if (lanes == 32) { launch(gat_aggregate_kernel<P, 32, H>, 32); return GTA_OK; }
+  } else {
+    switch (lanes) {
+      case 4: if (H <= 4) { launch(gat_aggregate_kernel<P, 4, H>, 4); return GTA_OK; } break;
+      case 8: if (H <= 8) { launch(gat_aggregate_kernel<P, 8, H>, 8); return GTA_OK; } break;
+      case 16: launch(gat_aggregate_kernel<P, 16, H>, 16); return GTA_OK;
+      case 32: launch(gat_aggregate_kernel<P, 32, H>, 32); return GTA_OK;
+    }
   }
   return GTA_ERR_UNSUPPORTED;
 }
@@ -729,7 +733,8 @@ static int gat_aggregate_impl(const char* who, const int32_t* items_, int64_t nu
     if constexpr (sizeof(T) == 4) {
       rc = gat_run<F32x4>(who, heads, st, wl, ex, el, er, lder, slope, z, ldz, out, ldo, f, epilogue, rowmax, rowsum,
                           er_stats, stats_pitch, col_block);
-    } else if (f <= 128) {
+    } else if (f <= 128 || f % 8 != 0 || (f / heads) % 8 != 0) {
+      // 8-byte pieces of 4 features: every per-head width of whole pieces of 4, in windows of 128 above 128 features
       rc = gat_run<Bf16x4>(who, heads, st, wl, ex, el, er, lder, slope, z, ldz, out, ldo, f, epilogue, rowmax, rowsum,
                            er_stats, stats_pitch, col_block);
     } else {

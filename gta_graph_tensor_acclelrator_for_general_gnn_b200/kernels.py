@@ -209,9 +209,8 @@ def aggregate(g: DeviceGraph, x: torch.Tensor, w: torch.Tensor | None = None, ro
     f = int(x.shape[1])
     rows = sched.row_end - sched.row_begin
     o = out if out is not None else alloc_table(rows, f, x.device)
-    per = 16 // x.element_size()
-    if f % per and _ld(x) >= pad_row(f, x.dtype) and _ld(o) >= pad_row(f, x.dtype):
-        f = pad_row(f, x.dtype)      # run over the pad columns too (independent columns, never read back)
+    if f % 4 and _ld(x) >= pad4(f) and _ld(o) >= pad4(f):
+        f = pad4(f)      # whole 4-feature pieces: run over the pad columns too (independent columns, never read back)
     fn, fname = (lib.gta_aggregate_f32, "gta_aggregate_f32") if x.dtype == torch.float32 else \
         (lib.gta_aggregate_bf16, "gta_aggregate_bf16")
     wmode, wh = _cabi.W_NONE, 0
