@@ -20,6 +20,9 @@ namespace gta {
 //   weighted aggregate   6x8: 3.36 ms   8x8: 3.29   8x4: 3.29   10x4: 3.13   (48 registers, no spills)
 //   GAT staged (H <= 4)  6x8: 3.89 ms   7x8: 3.88   8x8: 3.75   8x4: 3.49   10x4: 4.11 (spills)
 // More resident warps beat a deeper unroll: the kernels wait on L2 latency (long scoreboard), not on issue.
+// The GAT kernel as it now stands (bound cache, next-item staging, single-exp chain fold) reverses that: bench.py reddit-gat,
+// NVIDIA B200 at 1000 W, kernel ms:  8x4: 3.87-3.92   7x4: 3.66   6x4: 3.77   7x8: 3.60   6x8: 3.73   8x8: 3.54-3.63
+// (36 B of spill stores at 64 registers); 8x8 is also fastest on reddit-heavy-gat and the bf16 table, outputs bitwise equal.
 #ifndef GTA_AGG_MINBLOCKS
 #define GTA_AGG_MINBLOCKS 10
 #endif
@@ -30,7 +33,7 @@ namespace gta {
 #define GTA_GAT_MINBLOCKS 8
 #endif
 #ifndef GTA_GAT_UNROLL
-#define GTA_GAT_UNROLL 4
+#define GTA_GAT_UNROLL 8
 #endif
 #ifndef GTA_LLH_MINBLOCKS
 #define GTA_LLH_MINBLOCKS 6
