@@ -5,7 +5,9 @@
 #include <cuda_bf16.h>
 #include <string.h>
 
+#include <mutex>
 #include <type_traits>
+#include <unordered_map>
 
 #include "common.cuh"
 #include "exchange.cuh"
@@ -202,7 +204,9 @@ __device__ __forceinline__ ItemCursor cursor_begin(const WorkList& wl, const Exc
     if (lane == 0) c.pending = atomicAdd(counter, kGroups);
     c.stride = 0;
   } else {
-    const int copy = ex.world > 1 ? ex.copy_ctas : 0;
+    // the copy CTAs of an exchange exist in feature window 0 only (they pull and return); in every other window
+    // all of gridDim.x are work CTAs, so the warps of each window cover [0, num_items) exactly once
+    const int copy = (ex.world > 1 && blockIdx.y == 0) ? ex.copy_ctas : 0;
     c.first = ((int32_t(blockIdx.x) - copy) * kAggWarps + int32_t(threadIdx.x >> 5)) * kGroups;
     c.stride = (int32_t(gridDim.x) - copy) * kAggWarps * kGroups;
     c.pending = 0;
@@ -400,15 +404,21 @@ static int lanes_for(int f, int kper = 4, int v = 1) {
   return l < 4 ? 4 : l;
 }
 
+// Cached per kernel, not per template argument K: K is the kernel's function-pointer type, which instances of one
+// parameter list share (aggregate_kernel with one piece per lane at 48 registers, 10 CTAs per SM, and with two pieces
+// at 64 registers, 8 per SM).  A count taken from another instance oversizes the grid, and static striding needs every
+// CTA of a window resident: a chain then waits on a CTA that cannot start.
 template <typename K>
 static int resident_ctas(K kernel) {
-  static int cached = 0;          // one static per kernel instantiation
-  if (cached > 0) return cached;
+  static std::mutex lock;
+  static std::unordered_map<const void*, int> cached;
+  std::lock_guard<std::mutex> hold(lock);
+  const auto hit = cached.find(reinterpret_cast<const void*>(kernel));
+  if (hit != cached.end()) return hit->second;
   int per_sm = 0, dev = 0, sms = kNumSMs;
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kAggThreads, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  cached = per_sm * sms;
-  return cached;
+  return cached[reinterpret_cast<const void*>(kernel)] = per_sm * sms;
 }
 
 // dynamic item fetch (take = 1) unless the caller asked for static striding (GTA_PHASE_STATIC: long lists of

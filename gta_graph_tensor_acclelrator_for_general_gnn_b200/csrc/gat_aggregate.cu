@@ -511,8 +511,11 @@ gat_aggregate_llh_kernel(const WorkList wl, const Exchange ex, const float* __re
       }
       __syncwarp();
     }
-    // who publishes a head's statistics: the first lane of the head (width >= 4), or the one lane that owns it
+    // who publishes a head's statistics: the first lane of the head (width >= 4), or the one lane that owns it.
+    // A chained item's successor folds max and sum from the statistics of ITS window, so there the first lane of the
+    // window saves them too: a head whose width does not divide 128 (f = 144, H = 12) starts in the window before.
     const bool head_leader = active && (HPL > 1 || (fo % d) == 0);
+    const bool window_leader = head_leader || (active && l == 0);
     const bool chained = have && it.w >= 0;
     chain_step<LANES>(flags, lane, it, chained,
         [&]() { return make_int2(__ldg(wl.row_slots + it.x), __ldg(wl.row_slots + it.x + 1)); },
@@ -540,7 +543,7 @@ gat_aggregate_llh_kernel(const WorkList wl, const Exchange ex, const float* __re
         [&](int slot) {
           float* part = wl.partials + int64_t(slot) * pstride;
           if (active) *reinterpret_cast<float4*>(part + fo) = acc;
-          if (head_leader) {
+          if (window_leader) {
 #pragma unroll
             for (int k = 0; k < HPL; ++k) {
               part[stats + head + k] = m[k];

@@ -318,8 +318,10 @@ def gat_aggregate(g: DeviceGraph, el: torch.Tensor, er: torch.Tensor, z: torch.T
                   want_stats: bool = False, block_events=None, bounded: bool = True, exchange=None):
     """GAT ops 3-13 in one pass: returns ``out`` or ``(out, rowmax, rowsum)``.  ``bounded`` shifts the softmax
     by the per-(row, column block) bound ``leaky(el + max er)`` where the block's er range allows it (see
-    ``gta_er_stats``); ``False`` or ``want_stats`` runs the online softmax with a running maximum.  ``exchange``
-    (a ``dist.Gate``): ``z`` / ``er`` are views of this step's gathered table of a fused exchange, see ``aggregate``."""
+    ``gta_er_stats``); ``want_stats`` runs the online softmax with a running maximum, and so does ``False`` without
+    an exchange.  ``exchange`` (a ``dist.Gate``): ``z`` / ``er`` are views of this step's gathered table of a fused
+    exchange, see ``aggregate``; the bound then comes from the er ranges the slot owners published with the step,
+    whatever ``bounded`` says, so only ``want_stats`` selects the online softmax there."""
     lib = _cabi.load()
     _require_cuda(el, er, z)
     if exchange is not None:

@@ -7,6 +7,7 @@ import pytest
 from conftest import assert_close_rowscale
 from oracle import gta_oracle as O
 from gta_graph_tensor_acclelrator_for_general_gnn_b200 import synthetic
+from test_gpu_exchange import assert_slots_hold, emulated, release, run_step
 
 pytestmark = pytest.mark.gpu
 
@@ -83,69 +84,79 @@ def test_fused_exchange_gat_emulated(world, heads):
     """The in-kernel exchange end to end on one GPU: per rank, GEMM straight into slot 0 of its table,
     gta_exchange_publish to every peer's signal block, then an aggregation launch whose first CTAs copy the
     peers' slots (here: other buffers of the same device) while the rest walk the work list behind the slot
-    gates.  Three steps exercise both table parities; every step must give the same bits and the oracle's values."""
+    gates.  Three steps on X, another X, X again exercise both table parities with data that changes: every step must
+    give the oracle's values for its own X, and step 3 the bits of step 1."""
     import torch
-    from gta_graph_tensor_acclelrator_for_general_gnn_b200 import dist as gdist, kernels
+    from gta_graph_tensor_acclelrator_for_general_gnn_b200 import kernels
     indptr, indices, full, xd, wd, ald, ard, host = _gat_case(h=heads)
     x, w, al, ar = host
     f = int(wd.shape[1])
-    ref = O.gat_layer(indptr, indices, x, w, al, ar)
-    zabs = np.abs(x).astype(np.float64) @ np.abs(w).astype(np.float64)
-    scale = O.segment_sum(O.head_broadcast(ref["alpha"], f) * zabs[indices], indptr)
-    parts = [gdist.make_partition(full, r, world) for r in range(world)]
-    exs = [gdist.FusedExchange(p, copy_ctas=8) for p in parts]
-    for ex in exs:
-        ex.emulate_with(exs)
+    x1 = np.random.default_rng(world * 10 + heads).standard_normal(x.shape, dtype=np.float32)
+    data = {0: (x, xd), 1: (x1, torch.from_numpy(x1).cuda())}
+    parts, exs = emulated(full, world, copy_ctas=8)
     outs = []
-    for step in range(3):
-        staged = []
-        for p, ex in zip(parts, exs):          # phase 1 on every rank: producer + publish
+    for step, d in enumerate((0, 1, 0)):
+        xs = data[d][1]
+
+        def produce(p, ex):
             zv, erv = ex.local_views(f, heads, "cuda")
-            z, el, er = kernels.gemm(xd[p.row_begin:p.row_end], wd, ald, ard, out=zv, er_out=erv)
+            z, el, er = kernels.gemm(xs[p.row_begin:p.row_end], wd, ald, ard, out=zv, er_out=erv)
             assert z.data_ptr() == zv.data_ptr() and er.data_ptr() == erv.data_ptr()
             zt, ert, gate = ex.gather_pair(z, er)
             assert gate.struct.step == step + 1 and gate.slot_rows == p.stride
-            staged.append((el, zt, ert, gate))
-        got = torch.cat([kernels.gat_aggregate(p.local, el, ert, zt, exchange=gate)      # phase 2: pull + reduce
-                         for p, (el, zt, ert, gate) in zip(parts, staged)])
-        torch.cuda.synchronize()
+            return (zt, ert), gate, el
+
+        def consume(p, tables, gate, el):          # pull + reduce
+            return kernels.gat_aggregate(p.local, el, tables[1], tables[0], exchange=gate)
+        res = run_step(parts, exs, produce, consume)
+        # after the launch every slot of every rank's table holds its owner's rows of this step (its owner's slot 0)
+        own = [tables[0][:p.rows] for p, (_, tables, _) in zip(parts, res)]
+        assert_slots_hold(parts, res, (torch.cat(own),), f"fused exchange world={world} H={heads} step={step + 1}")
+        got = torch.cat([o for o, _, _ in res])
         outs.append(got)
-        # after the launch every slot of every rank's table holds its owner's rows
-        for p, (_, zt, _, _) in zip(parts, staged):
-            for k in range(world):
-                q = p.owner_of(k)
-                assert torch.equal(zt[k * p.stride: k * p.stride + parts[q].rows], staged[q][1][:parts[q].rows])
-    assert torch.equal(outs[0], outs[1]) and torch.equal(outs[0], outs[2])
-    assert_close_rowscale(outs[0].cpu().numpy(), ref["Y"], scale, what=f"fused exchange world={world} H={heads}")
+        ref = O.gat_layer(indptr, indices, data[d][0], w, al, ar)
+        zabs = np.abs(data[d][0]).astype(np.float64) @ np.abs(w).astype(np.float64)
+        scale = O.segment_sum(O.head_broadcast(ref["alpha"], f) * zabs[indices], indptr)
+        assert_close_rowscale(got.cpu().numpy(), ref["Y"], scale, what=f"fused exchange world={world} H={heads} step={step + 1}")
+    assert torch.equal(outs[0], outs[2])
+    release(exs)
 
 
 @pytest.mark.parametrize("world", [2, 8])
 def test_fused_exchange_gcn_emulated(world):
-    """Same for the weighted aggregate (GCN): gather_one, edge weights permuted into the local edge order."""
+    """Same for the weighted aggregate (GCN): gather_one, edge weights permuted into the local edge order; Z changes
+    from step to step."""
     import torch
-    from gta_graph_tensor_acclelrator_for_general_gnn_b200 import dist as gdist, graph, kernels
+    from gta_graph_tensor_acclelrator_for_general_gnn_b200 import graph, kernels
     n, e, f = 3000, 90000, 64
     g = synthetic.powerlaw_graph(n, e, seed=4, i0=3.0)
     indptr, indices, _ = O.csr_build(g.dst, g.src, n)
     full = graph.csr_from_coo(g.dst, g.src, n)
     rng = np.random.default_rng(2)
-    z = rng.standard_normal((n, f), dtype=np.float32)
+    zs = [rng.standard_normal((n, f), dtype=np.float32) for _ in range(2)]
     ew = synthetic.gcn_edge_norm(indptr, indices)
-    zd, ewd = torch.from_numpy(z).cuda(), torch.from_numpy(ew).cuda()
-    want = O.spmm(indptr, indices, ew, z)
-    scale = O.spmm(indptr, indices, np.abs(ew), np.abs(z))
-    parts = [gdist.make_partition(full, r, world) for r in range(world)]
-    exs = [gdist.FusedExchange(p, copy_ctas=4) for p in parts]
-    for ex in exs:
-        ex.emulate_with(exs)
-    for step in range(2):
-        staged = [ex.gather_one(zd[p.row_begin:p.row_end]) for p, ex in zip(parts, exs)]
-        outs = []
-        for p, (table, gate) in zip(parts, staged):
+    ewd = torch.from_numpy(ew).cuda()
+    parts, exs = emulated(full, world, copy_ctas=4)
+    outs = []
+    for step, d in enumerate((0, 1, 0)):
+        zd = torch.from_numpy(zs[d]).cuda()
+
+        def produce(p, ex):
+            table, gate = ex.gather_one(zd[p.row_begin:p.row_end])
+            return (table,), gate
+
+        def consume(p, tables, gate):
             e0, e1 = int(indptr[p.row_begin]), int(indptr[p.row_end])
-            outs.append(kernels.aggregate(p.local, table, p.permute_edges(ewd[e0:e1]), exchange=gate))
-        got = torch.cat(outs).cpu().numpy()
-        assert_close_rowscale(got, want, scale, what=f"fused GCN exchange world={world} step={step}")
+            return kernels.aggregate(p.local, tables[0], p.permute_edges(ewd[e0:e1]), exchange=gate)
+        res = run_step(parts, exs, produce, consume)
+        assert_slots_hold(parts, res, (zd,), f"fused GCN exchange world={world} step={step + 1}")
+        got = torch.cat([o for o, _, _ in res])
+        outs.append(got)
+        want = O.spmm(indptr, indices, ew, zs[d])
+        scale = O.spmm(indptr, indices, np.abs(ew), np.abs(zs[d]))
+        assert_close_rowscale(got.cpu().numpy(), want, scale, what=f"fused GCN exchange world={world} step={step + 1}")
+    assert torch.equal(outs[0], outs[2])
+    release(exs)
 
 
 def test_partition_from_coo_equals_make_partition():
@@ -213,33 +224,44 @@ def test_schedule_cut_points_equal_uniform_blocks():
 @pytest.mark.parametrize("world", [2, 4])
 def test_fused_exchange_bf16_tables_emulated(world):
     """bf16 storage mode across ranks: the IPC tables hold [Z bf16 | er fp32] rows (half the bytes of the pull), the GEMM
-    rounds Z into slot 0, the bf16 gather kernel reads the pulled slots.  Against the fp64 oracle at the mode's tolerance,
-    and against the single-GPU bf16 run at the fp32 tolerance (same stored values, other reduction order)."""
+    rounds Z into slot 0, the bf16 gather kernel reads the pulled slots.  X changes from step to step.  Against the fp64
+    oracle at the mode's tolerance, and against the single-GPU bf16 run at the fp32 tolerance (same stored values, other
+    reduction order)."""
     import torch
-    from gta_graph_tensor_acclelrator_for_general_gnn_b200 import dist as gdist, kernels
+    from gta_graph_tensor_acclelrator_for_general_gnn_b200 import kernels
     indptr, indices, full, xd, wd, ald, ard, host = _gat_case()
     x, w, al, ar = host
     f, heads = int(wd.shape[1]), int(ald.shape[1])
-    ref = O.gat_layer(indptr, indices, x, w, al, ar)
-    zabs = np.abs(x).astype(np.float64) @ np.abs(w).astype(np.float64)
-    scale = O.segment_sum(O.head_broadcast(ref["alpha"], f) * zabs[indices], indptr)
-    z1, el1, er1 = kernels.gemm(xd, wd, ald, ard, z_dtype=torch.bfloat16)
-    single = kernels.gat_aggregate(full, el1, er1, z1).cpu().numpy()
-    parts = [gdist.make_partition(full, r, world) for r in range(world)]
-    exs = [gdist.FusedExchange(p, copy_ctas=8) for p in parts]
-    for ex in exs:
-        ex.emulate_with(exs)
-    for step in range(2):
-        staged = []
-        for p, ex in zip(parts, exs):
+    x1 = np.random.default_rng(world).standard_normal(x.shape, dtype=np.float32)
+    data = {0: (x, xd), 1: (x1, torch.from_numpy(x1).cuda())}
+    parts, exs = emulated(full, world, copy_ctas=8)
+    outs = []
+    for step, d in enumerate((0, 1, 0)):
+        xh, xs = data[d]
+        ref = O.gat_layer(indptr, indices, xh, w, al, ar)
+        zabs = np.abs(xh).astype(np.float64) @ np.abs(w).astype(np.float64)
+        scale = O.segment_sum(O.head_broadcast(ref["alpha"], f) * zabs[indices], indptr)
+        z1, el1, er1 = kernels.gemm(xs, wd, ald, ard, z_dtype=torch.bfloat16)
+        single = kernels.gat_aggregate(full, el1, er1, z1).cpu().numpy()
+
+        def produce(p, ex):
             zv, erv = ex.local_views(f, heads, "cuda", torch.bfloat16)
             assert zv.dtype == torch.bfloat16 and erv.dtype == torch.float32
-            z, el, er = kernels.gemm(xd[p.row_begin:p.row_end], wd, ald, ard, out=zv, er_out=erv)
+            z, el, er = kernels.gemm(xs[p.row_begin:p.row_end], wd, ald, ard, out=zv, er_out=erv)
             zt, ert, gate = ex.gather_pair(z, er)
             assert gate.struct.row_bytes == 2 * f + 16 and zt.dtype == torch.bfloat16
-            staged.append((el, zt, ert, gate))
-        got = torch.cat([kernels.gat_aggregate(p.local, el, ert, zt, exchange=gate)
-                         for p, (el, zt, ert, gate) in zip(parts, staged)]).cpu().numpy()
+            return (zt, ert), gate, el
+
+        def consume(p, tables, gate, el):
+            return kernels.gat_aggregate(p.local, el, tables[1], tables[0], exchange=gate)
+        res = run_step(parts, exs, produce, consume)
+        own = [tables[0][:p.rows] for p, (_, tables, _) in zip(parts, res)]
+        assert_slots_hold(parts, res, (torch.cat(own),), f"bf16 exchange world={world} step={step + 1}")
+        got_t = torch.cat([o for o, _, _ in res])
+        outs.append(got_t)
+        got = got_t.cpu().numpy()
         bound = 2e-2 * np.abs(ref["Y"]) + 1e-2 * scale + 1e-30
         assert np.all(np.isfinite(got)) and np.max(np.abs(got - ref["Y"]) / bound) <= 1.0
-        assert_close_rowscale(got, single.astype(np.float64), scale, what=f"bf16 exchange world={world} step={step}")
+        assert_close_rowscale(got, single.astype(np.float64), scale, what=f"bf16 exchange world={world} step={step + 1}")
+    assert torch.equal(outs[0], outs[2])
+    release(exs)

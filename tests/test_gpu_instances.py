@@ -212,6 +212,7 @@ CASES = [
     (("gat", "f32", 48, 48), LLH(16, 4)),
     (("gat", "f32", 96, 6), LLH(32, 1)),
     (("gat", "f32", 256, 8), LLH(32, 1)),
+    (("gat", "f32", 144, 12), LLH(32, 1)),          # head 10 straddles the two 128-feature windows
     (("gat", "f32", 128, 64), LLH(32, 2)),
     (("gat", "f32", 128, 128), LLH(32, 4)),
     # edge sum (fp32): lanes = pieces of 4 features up to 32; which of edge / x are present picks the instance

@@ -374,6 +374,11 @@ def test_static_striding_is_the_same_reduction(T, monkeypatch, chunk, col_block)
     el16, er16 = _dev(T, rng.standard_normal((n, 16), dtype=np.float32)), _dev(T, rng.standard_normal((n, 16), dtype=np.float32))
     w = _dev(T, rng.random((g.num_edges, 1), dtype=np.float32))
     et = T.k.to_table(_dev(T, rng.standard_normal((g.num_edges, 128), dtype=np.float32)))
+    # widths just above one feature window: every kernel then runs a second window (blockIdx.y = 1) of the same cursor
+    gen = T.torch.Generator(device="cuda").manual_seed(12)
+    zw = T.torch.randn((n, 260), generator=gen, device="cuda")
+    el2, er2, el12, er12 = (T.torch.randn((n, h), generator=gen, device="cuda") for h in (2, 2, 12, 12))
+    w3 = T.torch.rand((g.num_edges, 3), generator=gen, device="cuda") + 0.1
     runs = {
         "aggregate": lambda: T.k.aggregate(dg, z, w, sched=sched),
         "aggregate 256 wide": lambda: T.k.aggregate(dg, z256, w, sched=sched),
@@ -383,6 +388,10 @@ def test_static_striding_is_the_same_reduction(T, monkeypatch, chunk, col_block)
         "gat bf16": lambda: T.k.gat_aggregate(dg, el, er, zb, sched=sched),
         "gat 16 heads": lambda: T.k.gat_aggregate(dg, el16, er16, z, sched=sched),
         "edge sum": lambda: T.k.aggregate_edge_sum(dg, et, z, z, T.cabi.UN_RELU, sched=sched),
+        "aggregate 260 wide unweighted": lambda: T.k.aggregate(dg, zw, sched=sched),
+        "aggregate 132 wide per-head": lambda: T.k.aggregate(dg, zw[:, :132], w3, sched=sched),
+        "gat 136 wide 2 heads": lambda: T.k.gat_aggregate(dg, el2, er2, zw[:, :136], sched=sched),
+        "gat 144 wide 12 heads": lambda: T.k.gat_aggregate(dg, el12, er12, zw[:, :144], sched=sched),
     }
     dynamic = {k: f().clone() for k, f in runs.items()}
     monkeypatch.setattr(T.k, "STATIC_MIN_ITEMS", 0)
