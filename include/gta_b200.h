@@ -201,7 +201,11 @@ int gta_schedule_build_cuts(const int64_t* indptr, const int32_t* indices, int64
  * Optional fused GAT ops 1,2 (genGraphOP.py:50-51): el = Z.Al, er = Z.Ar with Al,Ar [F,H]
  * row-major dense; pass NULL to skip.  el is dense [N,H]; er has row stride `lder` elements
  * (0 = dense), so a partitioned run can write z and er straight into its slot of the gathered
- * [F | H] source table.  fp32 in / fp32 out, fp32-accurate (rtol 1e-5).
+ * [F | H] source table.  fp32 in / fp32 out.  Error bound, with s = sum_k |x_k w_k|:
+ * FFMA path |z - z64| <= 1e-5 |z64| + 1e-5 s.  tcgen05 path: the same plus 2^-26 K s, because
+ * its fp32 accumulator loses about 1.2e-8 K relative on same-sign data (measured on an NVIDIA
+ * B200 at 1000 W: 7.8e-6 at K = 602, 1.7e-5 at K = 1433, 4.7e-5 at K = 4096; FFMA 1.5e-6,
+ * 2.3e-6, 3.8e-6).  With terms of mixed sign the error cancels and both paths hold 1e-5.
  * ------------------------------------------------------------------------------------ */
 /* `workspace` (gta_gemm_workspace(k,f) bytes, 128-byte aligned) holds the hi/lo TF32 split of W
  * for the tensor-core kernel; without it the call takes the FFMA kernel. */

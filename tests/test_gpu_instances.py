@@ -67,8 +67,9 @@ def library_instances(path: str = _cabi.LIB_PATH) -> set:
         return {_from_mangled(*m) for m in _MANGLED.findall(fh.read())}
 
 
-def launched(fn):
-    """Run fn() under the profiler (CUDA activity only): returns (fn's result, set of family instances that ran)."""
+def launched(fn, parse=kernel_instance):
+    """Run fn() under the profiler (CUDA activity only): returns (fn's result, set of instances that ran), an
+    instance being whatever parse() makes of a kernel name (None: not one of the kernels looked for)."""
     import torch
     from torch.profiler import ProfilerActivity, profile
     torch.cuda.synchronize()
@@ -77,7 +78,7 @@ def launched(fn):
         torch.cuda.synchronize()
     names = [e.name for e in prof.events()]
     assert names, "the profiler recorded no kernels: which instance ran cannot be told"
-    return result, {inst for inst in map(kernel_instance, names) if inst is not None}
+    return result, {inst for inst in map(parse, names) if inst is not None}
 
 
 # ---- the case table ------------------------------------------------------------------------------------------------
