@@ -201,7 +201,9 @@ int gta_csr_build(const int32_t* dst, const int32_t* src, int64_t num_edges, int
                   int64_t* indptr, int32_t* indices, int64_t* perm, void* workspace,
                   size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  GTA_REQUIRE(num_nodes > 0 && num_nodes < (int64_t(1) << 31), "gta_csr_build: num_nodes out of range");
+  // num_nodes = 0 is the local graph of a rank whose destination range is empty: indptr = [0], and any edge names a
+  // destination outside the graph, which the bad-id count below refuses
+  GTA_REQUIRE(num_nodes >= 0 && num_nodes < (int64_t(1) << 31), "gta_csr_build: num_nodes out of range");
   GTA_REQUIRE(num_edges >= 0 && num_edges < (int64_t(1) << 31), "gta_csr_build: num_edges must be < 2^31");
   GTA_REQUIRE(indptr && (num_edges == 0 || (dst && src && indices)), "gta_csr_build: null pointer");
   CsrWorkspace w = carve_csr(workspace, num_edges, num_nodes);

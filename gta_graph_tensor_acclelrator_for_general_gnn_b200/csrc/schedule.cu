@@ -175,12 +175,13 @@ static int schedule_build_impl(const int64_t* indptr, const int32_t* indices, in
   GTA_REQUIRE(indptr && items && row_slots && h_counts && workspace, "gta_schedule_build: null pointer");
   GTA_REQUIRE(chunk >= 32, "gta_schedule_build: chunk must be >= 32");
   GTA_REQUIRE(row_end >= row_begin, "gta_schedule_build: negative row range");
-  GTA_REQUIRE(n_cb == 1 || indices, "gta_schedule_build: column blocking needs the CSR indices");
   const int64_t rows = row_end - row_begin;
   h_counts[0] = h_counts[1] = 0;
   if (h_block_begin)
     for (int32_t cb = 0; cb <= n_cb; ++cb) h_block_begin[cb] = 0;
+  // no rows (a rank whose destination range is empty): no items, and the indices of its 0 edges may be NULL
   if (rows == 0) return GTA_OK;
+  GTA_REQUIRE(n_cb == 1 || indices, "gta_schedule_build: column blocking needs the CSR indices");
   const size_t need = gta_schedule_workspace(rows, ws_sources, ws_col_block);
   if (workspace_bytes < need) {
     set_error("gta_schedule_build: workspace %zu < required %zu", workspace_bytes, need);

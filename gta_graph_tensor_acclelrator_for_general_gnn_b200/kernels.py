@@ -343,8 +343,10 @@ def gat_aggregate(g: DeviceGraph, el: torch.Tensor, er: torch.Tensor, z: torch.T
     partials, chain = _chain_state(_gat_ws, sched.num_slots, stride, f, z.device)
     col_block = sched.col_block if sched.num_blocks > 1 else 0
     # with chunk events the table is still arriving: its er range is not known before the launch
-    # (with an exchange the slot owners publish their er range and the kernel reads it from the signal block)
-    stats = er_stats(er, col_block) if bounded and not want_stats and block_events is None and exchange is None else None
+    # (with an exchange the slot owners publish their er range and the kernel reads it from the signal block);
+    # an empty work list (a rank without rows) launches nothing at all
+    stats = er_stats(er, col_block) if (bounded and not want_stats and block_events is None and exchange is None
+                                        and sched.num_items > 0) else None
 
     fn, fname = (lib.gta_gat_aggregate_f32, "gta_gat_aggregate_f32") if z.dtype == torch.float32 else \
         (lib.gta_gat_aggregate_bf16, "gta_gat_aggregate_bf16")

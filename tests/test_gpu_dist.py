@@ -1,6 +1,6 @@
 """Destination-partitioned execution, all ranks emulated on ONE GPU.  No kernel here waits on a kernel that
 has not been launched: every rank's producer + publish runs first, then every rank's aggregation -- whose copy
-CTAs then find all peers ready.  (Real multi-GPU runs: bench.py --gpus N, which checks parity itself.)"""
+CTAs then find all peers ready.  (Real ranks, one GPU each: test_gpu_multiprocess.py.)"""
 import numpy as np
 import pytest
 

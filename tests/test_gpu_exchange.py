@@ -10,7 +10,7 @@ offsets far enough apart that a stale bound overflows or underflows exp, make su
 Every compiled aggregate and GAT instance (the case table of test_gpu_instances.py) runs through a world-4 exchange,
 whose slot groups [[0], [1], [2, 3]] give items that span two slots; then the partition edges (world sizes, one copy
 CTA, ranks without rows, 3 and 32 heads, a wide er range beside narrow ones); then static striding on widths that
-need a second feature window.  (Real multi-GPU runs: bench.py --gpus N, which checks parity itself.)
+need a second feature window.  (Real ranks, one GPU each: test_gpu_multiprocess.py.)
 """
 import types
 import zlib
@@ -291,10 +291,7 @@ EDGES = {
     "heads32": (4, 0, "crafted", 32, False),
     "wide-er": (4, 0, "crafted", None, True),
 }
-#: a rank whose edge-balanced range is empty cannot build its local CSR yet (gta_csr_build takes at least one node):
-#: the partition fails loudly at setup.  Strict, so that the case is switched on once such ranks are supported.
-NO_ROWS = pytest.mark.xfail(raises=_cabi.GtaError, strict=True, reason="a rank without rows has no local CSR")
-EDGE_RUNS = [pytest.param(kind, v, id=f"{kind}-{v}", marks=[NO_ROWS] if v == "empty-ranks" else [])
+EDGE_RUNS = [pytest.param(kind, v, id=f"{kind}-{v}")
              for kind in ("gat-f32", "gat-bf16", "gcn") for v in EDGES
              if not (kind != "gat-f32" and EDGES[v][3] is not None)          # bf16 GAT: 1, 2 or 4 heads; GCN: no heads
              and not (kind == "gcn" and EDGES[v][4])]

@@ -78,6 +78,37 @@ def test_csr_build_duplicates_and_empty(T):
     assert np.array_equal(empty.indptr.cpu().numpy(), np.zeros(6, np.int64))
 
 
+def test_graph_without_rows(T):
+    """The local graph of a rank whose edge-balanced range is empty: 0 nodes give indptr = [0] and a work list of 0
+    items, and the calls of a step on it (GEMM over 0 rows, aggregations over 0 items, with the NULL data pointer of an
+    empty edge-weight tensor) return empty outputs without a launch.  An edge into a 0-node graph is refused."""
+    torch, k = T.torch, T.k
+    g = T.graph.csr_from_coo(np.zeros(0, np.int32), np.zeros(0, np.int32), 0, want_perm=True)
+    assert g.num_rows == 0 and g.num_edges == 0 and g.indptr.cpu().tolist() == [0]
+    assert g.schedule().num_items == 0 and g.schedule(col_cuts=(8, 16)).num_items == 0
+    with pytest.raises(T.cabi.GtaError, match="outside"):
+        T.graph.csr_from_coo(np.zeros(1, np.int32), np.zeros(1, np.int32), 0)
+    g.num_sources = 16
+    lib = T.cabi.load()
+    x = torch.zeros((0, 64), device="cuda")
+    w = torch.randn(64, 32, device="cuda")
+    al, ar = torch.randn(32, 4, device="cuda"), torch.randn(32, 4, device="cuda")
+    table = k.alloc_table(16, 32, "cuda", zero=True)
+    er_table = torch.zeros((16, 4), device="cuda")
+    torch.cuda.synchronize()
+    lib.gta_launch_count_reset()
+    z, el, er = k.gemm(x, w, al, ar)
+    assert z.shape == (0, 32) and el.shape == (0, 4) and er.shape == (0, 4)
+    ew = torch.empty((0, 1), device="cuda")
+    assert ew.data_ptr() == 0          # what a rank without edges hands the weighted aggregate
+    assert k.aggregate(g, table, ew).shape == (0, 32)
+    assert k.aggregate(g, table).shape == (0, 32)
+    assert k.gat_aggregate(g, el, er_table, table).shape == (0, 32)
+    out, rowmax, rowsum = k.gat_aggregate(g, el, er_table, table, want_stats=True)
+    assert out.shape == (0, 32) and rowmax.shape == (0, 4) and rowsum.shape == (0, 4)
+    assert int(lib.gta_launch_count()) == 0
+
+
 def test_tile_nnz_against_reference_tables(T, golden_dir):
     import os
     for tag in ("g300", "g97"):
